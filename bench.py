@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- flow records/s through EWMA throughput-anomaly detection (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one complete TAD job (stage A filter/reduce, group, time sort, stddev_samp, EWMA,
 anomaly compaction) over one synthetic flow table of BASELINE.json configs[1]: 100M records /
@@ -134,6 +134,35 @@ def sample_mask(src_ip, dst_ip, frac):
     return h < max(1, int(frac * (1 << 20)))
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_sample(res, result_rows):
+    """The rows of `res` (one job's result columns, or one rank's share of them) that --dump-outputs keeps: every row when
+    the whole result (`result_rows` rows over all ranks) fits half of DUMP_BYTES as float64, else the connections that
+    sample_mask selects with the largest power-of-two fraction that does.  Returns (rows, fraction)."""
+    frac = 1.0
+    while result_rows * frac * 8 * len(res) > DUMP_BYTES / 2:
+        frac /= 2
+    if frac < 1.0:
+        m = sample_mask(res["src_ip"], res["dst_ip"], frac)
+        res = {k: v[m] for k, v in res.items()}
+    return res, frac
+
+
+def write_outputs(out_dir, res, result_rows, frac):
+    """DIR/<column>.npy, float64 (every result column is FP64 or an integer below 2^53), rows in canonical (key, flowEnd)
+    order so that two builds compare element for element; cut to DUMP_BYTES in that order."""
+    import numpy as np
+    from oracle import tad_oracle
+    res = tad_oracle.canonicalize(res)
+    keep = min(len(res["flow_end"]), DUMP_BYTES // (8 * len(res)))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in res.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[:keep].astype(np.float64))
+    return {"dir": out_dir, "rows": keep, "result_rows": result_rows, "connection_fraction": frac, "dtype": "float64"}
+
+
 def parity_check(eng, dcols, cols_t, algo, global_rows, total_series, dist, rank, world, want_connections=3000):
     """One more (untimed) job on the bench table; the connections of a hash-selected sample are cross-checked bit for bit
     against the CPU oracle (the checker; tests/test_gpu_full_size.py does the same): the input rows of the sample are
@@ -262,6 +291,11 @@ def run_reference(args):
         cols, ns, npts = c_oracle.run_job(t, algo=0, threads=cores)
     dt = (time.perf_counter() - t0) / args.steps
     v = rows / dt
+    outputs = None
+    if args.dump_outputs:
+        n = len(cols["flow_end"])
+        sub, frac = dump_sample(cols, n)
+        outputs = write_outputs(args.dump_outputs, sub, n, frac)
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "records/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
@@ -276,7 +310,7 @@ def run_reference(args):
                              rows, cores, ns, npts),
                          "python_port_1core": python_port_rate(args.points)},
         "e2e": {"value": v, "unit": "records/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-        "gpu_launches": 0}))
+        "gpu_launches": 0, **({"outputs": outputs} if outputs else {})}))
 
 
 def side_run(eng, dev, algo, series, points, steps, warmup, name):
@@ -456,18 +490,39 @@ def run_ours(args):
     sampler.mark_begin()
     t0 = time.perf_counter()
     dev_ms, phase, launches, result_rows = 0.0, {}, 0, 0
-    for _ in range(args.steps):
+    last = None
+    for i in range(args.steps):
         job, st = step(dcols)
         dev_ms += st["device_ms"]
         launches += st["gpu_launches"]
         result_rows = st["result_rows"]
         for k, v in st["phase_ms"].items():
             phase[k] = phase.get(k, 0.0) + v
-        job.release()
+        if args.dump_outputs and i == args.steps - 1:
+            last = job                   # its rows are fetched once the clock has stopped
+        else:
+            job.release()
     barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
     sampler.mark_end()
     clocks = sampler.stop() if rank == 0 else None
+
+    # ---- --dump-outputs: the result rows of the last timed step (all ranks' shares, sampled alike) ----------------------
+    outputs = None
+    if last is not None:
+        res = last.result()
+        last.release()
+        n = torch.tensor([len(res["flow_end"])], device=dev, dtype=torch.int64)
+        if dist is not None:
+            dist.all_reduce(n)
+        res, frac = dump_sample(res, int(n[0]))
+        if dist is not None:
+            box = [None] * world if rank == 0 else None
+            dist.gather_object(res, box, dst=0)
+            if rank == 0:
+                res = {k: np.concatenate([b[k] for b in box]) for k in res}
+        if rank == 0:
+            outputs = write_outputs(args.dump_outputs, res, int(n[0]), frac)
     stats = torch.tensor([dev_ms / args.steps, wall_ms / args.steps], device=dev, dtype=torch.float64)
     if dist is not None:
         dist.all_reduce(stats, op=dist.ReduceOp.MAX)
@@ -488,7 +543,7 @@ def run_ours(args):
         if rank == 0:
             print(json.dumps({"value": total_rows / (ms_dev * 1e-3), "ms_per_step": ms_dev, "wall_ms_per_step": ms_wall,
                               "phase_ms": {k: v / args.steps for k, v in phase.items()}, "parity": parity,
-                              "note": "profiling run"}))
+                              "note": "profiling run", **({"outputs": outputs} if outputs else {})}))
         eng.close()
         if dist is not None:
             dist.destroy_process_group()
@@ -581,6 +636,8 @@ def run_ours(args):
             "phase_ms": per, "result_rows": result_rows, "clocks": clocks,
         }
         line["parity"] = parity
+        if outputs:
+            line["outputs"] = outputs
         line["phase_ms_meaning"] = {
             "h2d": "host->device column copies, with the partition kernels that run chunk by chunk behind them (0 for device-resident input)",
             "exchange": "several GPUs: gather of the peers' arrival counters (rows are pulled inside `group`); exact partition: exposed NCCL all-to-all",
@@ -653,7 +710,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs: skip the host-buffer leg")
     ap.add_argument("--no-pipelined", action="store_true", help="skip the two-jobs-in-flight e2e figure")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result rows of the last timed step as DIR/<column>.npy (float64, canonical row order, "
+                         "at most 64 MB: above that a fixed hash-selected subset of the connections)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

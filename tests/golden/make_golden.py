@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Generate the committed golden fixtures from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs the reference source tree (``THEIA_REFERENCE_ROOT``, see oracle/ref_loader.py):
 
     python tests/golden/make_golden.py
 
@@ -16,6 +16,8 @@ Writes
       called with ``decimal.Decimal`` elements as Spark hands them over
       (``Decimal(38,18)``, anomaly_detection.py:488).  scikit-learn here is 1.9.0
       (the reference pins 1.3.0); numpy 2.3.5.
+  tests/golden/udf_cases_oracle_stddev.json -- heavy-tailed seeded series and the outputs of the same
+      three reference UDFs when they are handed the oracle's own stddev_samp.
 
 The fixtures travel to the GPU box; the reference tree does not.
 """
@@ -66,6 +68,21 @@ def series_bank():
     return bank
 
 
+def oracle_stddev_cases(ad):
+    """Series with rare 300x spikes; the reference UDFs are handed the oracle's restatement of the job's stddev_samp."""
+    from oracle import tad_oracle
+    rng = np.random.default_rng(99)
+    cases = []
+    for n in (1, 2, 7, 11, 12, 40, 90):
+        vals = [int(x) for x in np.maximum(np.rint(4e9 + rng.normal(0, 4e6, n) * rng.choice([1, 1, 1, 300], n)), 1)]
+        dec = [Decimal(v) for v in vals]
+        sd = tad_oracle.stddev_samp(vals)
+        cases.append({"values": vals, "stddev": sd, "ewma": [float(e) for e in ad.calculate_ewma(dec)],
+                      "ewma_flags": [bool(b) for b in ad.calculate_ewma_anomaly(dec, sd)],
+                      "dbscan_flags": [bool(b) for b in ad.calculate_dbscan_anomaly(dec, sd)]})
+    return cases
+
+
 def main():
     ad = load_reference_job()
     with open(os.path.join(HERE, "reference_test_vectors.json"), "w") as f:
@@ -85,6 +102,12 @@ def main():
                    "reference_commit": "bc06ff0afe05c984f2efc7a53e68e8f152914c3e",
                    "cases": cases}, f)
     print("wrote %d udf cases" % len(cases))
+    cases = oracle_stddev_cases(ad)
+    with open(os.path.join(HERE, "udf_cases_oracle_stddev.json"), "w") as f:
+        json.dump({"generator": "tests/golden/make_golden.py",
+                   "reference_commit": "bc06ff0afe05c984f2efc7a53e68e8f152914c3e",
+                   "cases": cases}, f)
+    print("wrote %d oracle-stddev udf cases" % len(cases))
     # the reference's 12 SQL-generation cases (anomaly_detection_test.py:46-195): inputs + expected SQL text
     import importlib
     tmod = importlib.import_module("anomaly_detection_test")

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
              "vs_baseline", "dtype", "data", "config", "e2e", "gpu_launches"}
@@ -42,6 +44,50 @@ def test_reference_arm_runs_on_cpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
                           "--ref-series", "100"], capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def _dumped(out_dir):
+    import numpy as np
+    return {f[:-4]: np.load(os.path.join(out_dir, f)) for f in os.listdir(out_dir)}
+
+
+def _oracle_rows_of_bench_table(series, points):
+    sys.path.insert(0, ROOT)
+    import bench
+    from tests.util import oracle_rows
+    return oracle_rows(bench.bench_table_numpy(series, points), "EWMA")[0]
+
+
+def test_reference_arm_dumps_its_outputs(tmp_path):
+    from tests.util import EXACT_COLS, SCORE_COLS, assert_same_rows
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                          "--series", "300", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads(out.stdout.strip().splitlines()[-1])
+    got = _dumped(tmp_path)
+    assert set(got) == set(EXACT_COLS + SCORE_COLS) and all(v.dtype.name == "float64" for v in got.values())
+    assert d["outputs"]["rows"] == d["outputs"]["result_rows"] == len(got["flow_end"]) > 0
+    assert_same_rows(got, _oracle_rows_of_bench_table(300, 100), what="dumped reference outputs")
+
+
+@pytest.mark.gpu
+def test_gpu_arm_times_steps_jobs_and_dumps_the_last_one(tmp_path):
+    """--steps K times K jobs; --dump-outputs writes the rows the last of them returned, which are the oracle's."""
+    from tests.util import assert_same_rows
+    lines = {}
+    for k in (1, 3):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--series", "3000", "--steps", str(k), "--warmup", "1",
+                              "--no-cpu", "--no-sides", "--no-pipelined", "--no-parity", "--dump-outputs", str(tmp_path / str(k))],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines[k] = json.loads(out.stdout.strip().splitlines()[-1])
+    assert lines[1]["steps"] == 1 and lines[3]["steps"] == 3
+    assert lines[3]["gpu_launches"] == 3 * lines[1]["gpu_launches"] > 0
+    want = _oracle_rows_of_bench_table(3000, 100)
+    for k in (1, 3):
+        o = lines[k]["outputs"]
+        assert o["rows"] == o["result_rows"] == lines[k]["result_rows"]
+        assert_same_rows(_dumped(tmp_path / str(k)), want, what="dumped outputs, --steps %d" % k)
 
 
 def test_sample_mask_is_the_same_subset_for_torch_and_numpy_columns():

@@ -2,19 +2,20 @@
 (plugins/anomaly-detection/anomaly_detection_test.py:199-402, committed as
 tests/golden/reference_test_vectors.json), (ii) outputs of the unmodified reference UDFs on
 seeded series (tests/golden/udf_cases.json, made by tests/golden/make_golden.py), and
-(iii) when the reference tree is present (build container), the live reference UDFs."""
+(iii) outputs of the same UDFs on heavy-tailed series when handed the oracle's own stddev
+(tests/golden/udf_cases_oracle_stddev.json, same generator)."""
 import json
 import os
-from decimal import Decimal
 
 import numpy as np
 import pytest
 
-from oracle import c_oracle, ref_loader, tad_oracle as o
+from oracle import c_oracle, tad_oracle as o
 
 G = os.path.join(os.path.dirname(__file__), "golden")
 REF = json.load(open(os.path.join(G, "reference_test_vectors.json")))
 CASES = json.load(open(os.path.join(G, "udf_cases.json")))["cases"]
+SD_CASES = json.load(open(os.path.join(G, "udf_cases_oracle_stddev.json")))["cases"]
 
 
 def test_reference_ewma_values_exact():
@@ -71,14 +72,11 @@ def test_c_port_matches_python(case):
     assert list(c_oracle.dbscan_series(v)) == case["dbscan_flags"]
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree only exists in the build container")
-def test_live_reference_udfs():
-    ad = ref_loader.load_reference_job()
-    rng = np.random.default_rng(99)
-    for n in (1, 2, 7, 11, 12, 40, 90):
-        vals = [int(x) for x in np.maximum(np.rint(4e9 + rng.normal(0, 4e6, n) * rng.choice([1, 1, 1, 300], n)), 1)]
-        dec = [Decimal(v) for v in vals]
+def test_recorded_reference_udfs():
+    for case in SD_CASES:
+        vals = case["values"]
         sd = o.stddev_samp(vals)
-        assert [float(e) for e in ad.calculate_ewma(dec)] == list(o.calculate_ewma(vals))
-        assert [bool(b) for b in ad.calculate_ewma_anomaly(dec, sd)] == list(o.calculate_ewma_anomaly(vals, sd))
-        assert [bool(b) for b in ad.calculate_dbscan_anomaly(dec, sd)] == list(o.calculate_dbscan_anomaly(vals))
+        assert sd == case["stddev"]
+        assert list(o.calculate_ewma(vals)) == case["ewma"]
+        assert list(o.calculate_ewma_anomaly(vals, sd)) == case["ewma_flags"]
+        assert list(o.calculate_dbscan_anomaly(vals)) == case["dbscan_flags"]
