@@ -8,9 +8,11 @@ mode = gpu : every rank runs its row shard of every case through the engine and 
                spread : rows shuffled over the ranks -> optimistic partition + peer pull (no histogram pass, no NCCL
                         exchange; asserted through phase_ms)
                skewed : two long connections sit on the last rank -> a slot overflows there, every rank falls back to
-                        the exact partition + NCCL all-to-all (chunked, overlapped)
-               xpull  : the skewed table with TAD_EXACT_PULL=1: the fallback's exact partition is pulled by the peers as well
-               nccl   : the spread table with the peer pull switched off (third engine)"""
+                        the exact partition, which the peers pull as well (no receive buffer)
+               xpull  : the skewed table on a fresh engine, two runs per algorithm (second engine)
+               nccl   : the spread table with the peer pull switched off: exact partition + NCCL all-to-all (chunked,
+                        overlapped) (third engine)
+               ncclskew : the skewed table on the third engine: the NCCL exchange with the spill path behind it"""
 import os
 import sys
 
@@ -82,7 +84,6 @@ def main():
                     np.savez(os.path.join(out_dir, "res_%s_%s_%d.npz" % (name, algo, rank)), **got)
         eng.close()
         # the exact partition pulled by the peers (no receive buffer): the skewed table overflows a slot, every rank falls back
-        os.environ["TAD_EXACT_PULL"] = "1"
         eng = engine(True)
         table = case_table("skewed")
         total = len(table["value"])
@@ -93,7 +94,6 @@ def main():
             assert st["phase_ms"]["hist"] > 0.0 and st["rows_kept"] == len(mine["value"])
             np.savez(os.path.join(out_dir, "res_xpull_%s_%d.npz" % (algo, rank)), **got)
         eng.close()
-        os.environ["TAD_EXACT_PULL"] = "0"
         eng = engine(False)
         table = case_table("spread")
         mine = sharding.shard_rows(table, rank, world)

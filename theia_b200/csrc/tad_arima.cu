@@ -11,7 +11,6 @@
 // Compute-bound FP64 (about n^2/2 Kalman steps x ~100 likelihood evaluations per series), so the
 // mapping is one WARP per series with one lane per prefix fit; the series lives in L1.
 #include <cfloat>
-#include <cstdlib>
 
 #include "tad_kernels.h"
 
@@ -540,8 +539,9 @@ __host__ __device__ bool lbfgs_advance(Lbfgs &s, double x[3], double f, const do
     return lbfgs_begin_iter(s, x);
 }
 
-// one fit, evaluated and advanced in place (host tests; the sequential device path)
-__host__ __device__ void arima_fit(const ArimaObj &o, double x[3])
+// one fit, evaluated and advanced in place, on the host: the numerical reference the CPU tests check through
+// tad_debug_arima_fit (arima_fit_sync_kernel runs the same steps per lane)
+void arima_fit(const ArimaObj &o, double x[3])
 {
     Lbfgs s;
     lbfgs_init(s);
@@ -589,38 +589,12 @@ __global__ void __launch_bounds__(128) arima_boxcox_kernel(const SeriesEntry *__
     lam[i] = finite ? l : NAN;                             // overflowing transform -> the series yields no rows
 }
 
-// one warp per series, one lane per prefix fit (t = 3 .. n-1); pred[] in Box-Cox space
-__global__ void __launch_bounds__(128) arima_fit_kernel(const SeriesEntry *__restrict__ entries, const uint32_t *__restrict__ offsets,
-                                                        const uint32_t *__restrict__ sbase, uint32_t B, uint32_t S,
-                                                        const double *__restrict__ yb, const double *__restrict__ lam,
-                                                        double *__restrict__ pred)
-{
-    const uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const uint32_t lane = threadIdx.x & 31;
-    if (i >= S) return;
-    if (isnan(lam[i])) return;
-    const SeriesEntry e = load_entry(entries, offsets, sbase, B, i);
-    const double *y = yb + e.off;
-    double *p = pred + e.off;
-    for (uint32_t t = lane; t < e.n; t += 32) {
-        if (t < 3) { p[t] = y[t]; continue; }             // train = first three points (:241,255)
-        ArimaObj o{y, t};
-        double u[3];
-        arima_start(o, u);
-        arima_fit(o, u);
-        double phi, theta, s2, fc = 0.0;
-        arima_transform(u, phi, theta, s2);
-        arima_loglike(o, phi, theta, s2, &fc);
-        p[t] = fc;
-    }
-}
-
-// Evaluation-synchronous variant: one warp per series; the prefix fits t = n-1 .. 3 form a job list that the lanes
-// work through dynamically (longest first, so the fits in flight have similar lengths).  Every round, all lanes that
-// hold a job evaluate the objective and its forward-difference gradient TOGETHER -- the same Kalman-filter loop, each lane
-// on its own prefix and parameters -- then each lane advances its own optimiser state (lbfgs_advance) to the next trial
-// point; a lane whose fit has ended writes its forecast and takes the next job.  Per fit the arithmetic is the same as
-// in arima_fit: only the scheduling differs.
+// Evaluation-synchronous fits, pred[] in Box-Cox space: one warp per series; the prefix fits t = n-1 .. 3 form a job list
+// that the lanes work through dynamically (longest first, so the fits in flight have similar lengths).  Every round, all
+// lanes that hold a job evaluate the objective and its forward-difference gradient TOGETHER -- the same Kalman-filter loop,
+// each lane on its own prefix and parameters -- then each lane advances its own optimiser state (lbfgs_advance) to the next
+// trial point; a lane whose fit has ended writes its forecast and takes the next job.  Per fit the arithmetic is the same
+// as in arima_fit: only the scheduling differs.
 __global__ void __launch_bounds__(128) arima_fit_sync_kernel(const SeriesEntry *__restrict__ entries, const uint32_t *__restrict__ offsets,
                                                              const uint32_t *__restrict__ sbase, uint32_t B, uint32_t S,
                                                              const double *__restrict__ yb, const double *__restrict__ lam,
@@ -774,14 +748,8 @@ cudaError_t launch_detect_arima(cudaStream_t st, const SeriesEntry *entries, con
     if (fit) {
         arima_boxcox_kernel<<<(S + 127) / 128, 128, 0, st>>>(entries, offsets, sbase, B, S, csr_v, scratch_y, scratch_lam);
         const uint64_t threads = (uint64_t)S * 32;
-        static int mode = -1;                      // TAD_ARIMA_MODE: 1 = evaluation-synchronous fits, 0 = one independent fit per lane
-        if (mode < 0) { const char *ev = getenv("TAD_ARIMA_MODE"); mode = ev ? atoi(ev) : 1; }
-        if (mode == 1)
-            arima_fit_sync_kernel<<<(uint32_t)((threads + 127) / 128), 128, 0, st>>>(entries, offsets, sbase, B, S, scratch_y,
-                                                                                    scratch_lam, scratch_pred);
-        else
-            arima_fit_kernel<<<(uint32_t)((threads + 127) / 128), 128, 0, st>>>(entries, offsets, sbase, B, S, scratch_y, scratch_lam,
-                                                                               scratch_pred);
+        arima_fit_sync_kernel<<<(uint32_t)((threads + 127) / 128), 128, 0, st>>>(entries, offsets, sbase, B, S, scratch_y,
+                                                                                scratch_lam, scratch_pred);
     }
     constexpr int NT = 128;
     detect_arima_kernel<NT><<<(S + NT - 1) / NT, NT, 0, st>>>(entries, offsets, sbase, B, S, csr_v, csr_t, scratch_pred,

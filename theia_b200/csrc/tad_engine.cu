@@ -180,11 +180,8 @@ struct tad_ctx {
     // exported buffer (arrival counters in front, slots behind), the peers map it (CUDA IPC) and the owner's group kernel
     // pulls its bucket segments over NVLink -- no histogram pass, no all-to-all, no receive buffer.
     int peer_pull = 1;                              // TAD_PEER_PULL=0: always the exact partition + NCCL all-to-all
-    GroupStreams gstreams{};                        // side streams of the group phase (capacity classes run concurrently)
-    int group_concurrent = 0;                       // TAD_GROUP_CONCURRENT=1
     int sort_classes = 0;                           // TAD_SORT_CLASSES=1: capacity-class bucket lists sorted by bucket before the group phase
     DevBuf sortb;
-    int exact_pull = 0;                             // TAD_EXACT_PULL=1: the exact partition is pulled by the peers too (no receive buffer)
     size_t x_budget = 72ull << 30;                  // largest exported slot buffer (TAD_SLOT_BUDGET_GB); beyond it: exact partition
     DevBuf xbuf;                                    // exported: [counters: B x u32, padded][slots: B x slot x Row32]
     void *peer_x[kMaxRanks]{};                      // peers' xbuf mapped into this process
@@ -700,7 +697,7 @@ void run_job(tad_ctx *ctx, tad_job *job)
         // longer than the scatter it could hide behind and the extra segments cost the group kernel more than is won
         // With peer pull (default) the exact partition is written into the EXPORTED buffer and the owners' group kernels read
         // their segments straight out of the peers' copies: no receive buffer, no all-to-all (and no chunking: K = 1).
-        const bool pull = ctx->peer_pull != 0 && ctx->exact_pull != 0;
+        const bool pull = ctx->peer_pull != 0;
         const int K = pull ? 1 : (R >= ctx->exchange_min_rows && (world == 2 || ctx->exchange_chunks_forced)) ? ctx->exchange_chunks : 1;
         auto xlo = [&](int cidx) -> uint64_t {
             if (cidx <= 0) return 0;
@@ -846,8 +843,7 @@ void run_job(tad_ctx *ctx, tad_job *job)
             for (int k = 0; k < 3; k++)
                 if (n_cls[k] > 1) { CU(sort_bucket_list(st, cls_list + (size_t)k * Bl, n_cls[k], bits, ctx->sortb.p, ctx->sortb.cap)); launches += 3; }
         }
-        CU(launch_group(st, seg, entries, offsets, Bl, logB, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb, sp.reducer, &l,
-                        ctx->group_concurrent ? &ctx->gstreams : nullptr));
+        CU(launch_group(st, seg, entries, offsets, Bl, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb, sp.reducer, &l));
         launches += l;
     }
     mark(TAD_PHASE_GROUP);
@@ -1104,17 +1100,9 @@ int tad_init(const tad_config *cfg, tad_ctx **out)
     // defaults = the fastest measured configuration per world size (DESIGN.md section 6): peer pull everywhere, the exact fallback
     // pulled as well, capacity-class lists sorted by bucket from 4 ranks on (locality of the small remote reads)
     ctx->peer_pull = 1;
-    ctx->exact_pull = 1;
     ctx->sort_classes = cfg->world_size >= 4 ? 1 : 0;
     if (const char *e = getenv("TAD_PEER_PULL")) ctx->peer_pull = atoi(e);
-    if (const char *e = getenv("TAD_EXACT_PULL")) ctx->exact_pull = atoi(e);
     if (const char *e = getenv("TAD_SORT_CLASSES")) ctx->sort_classes = atoi(e);
-    if (const char *e = getenv("TAD_GROUP_CONCURRENT")) ctx->group_concurrent = atoi(e);
-    for (int i = 0; ok && i < 2; i++) {
-        ok = cudaStreamCreateWithFlags(&ctx->gstreams.aux[i], cudaStreamNonBlocking) == cudaSuccess;
-        ok = ok && cudaEventCreateWithFlags(&ctx->gstreams.join[i], cudaEventDisableTiming) == cudaSuccess;
-    }
-    ok = ok && cudaEventCreateWithFlags(&ctx->gstreams.fork, cudaEventDisableTiming) == cudaSuccess;
     if (const char *e = getenv("TAD_SLOT_BUDGET_GB")) ctx->x_budget = (size_t)strtoull(e, nullptr, 10) << 30;
     if (const char *e = getenv("TAD_EXCHANGE_MIN_ROWS")) ctx->exchange_min_rows = strtoull(e, nullptr, 10);
     if (getenv("TAD_EXCHANGE_CHUNKS")) ctx->exchange_chunks_forced = true;
@@ -1175,11 +1163,6 @@ void tad_shutdown(tad_ctx *ctx)
     if (ctx->start_ev) cudaEventDestroy(ctx->start_ev);
     for (int i = 0; i <= kMaxXChunks; i++)
         if (ctx->x_ev[i]) cudaEventDestroy(ctx->x_ev[i]);
-    for (int i = 0; i < 2; i++) {
-        if (ctx->gstreams.join[i]) cudaEventDestroy(ctx->gstreams.join[i]);
-        if (ctx->gstreams.aux[i]) cudaStreamDestroy(ctx->gstreams.aux[i]);
-    }
-    if (ctx->gstreams.fork) cudaEventDestroy(ctx->gstreams.fork);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;

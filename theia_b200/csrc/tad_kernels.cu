@@ -9,7 +9,7 @@
 //                  key, O(n) bucket-sort of each series by flowEndSeconds, reduce duplicates,
 //                  write per-series arrays + series entries                   reads 32, writes 12 B/row
 //   sscan    (K3b) exclusive scan of series-per-bucket
-//   detect   (K4)  one thread per series out of a TMA-staged span: stddev_samp (Welford,
+//   detect   (K4)  one thread per series straight out of csr_v: stddev_samp (Welford,
 //                  sequential FP64), EWMA / DBSCAN score + flag, queued emission  reads 8-12 B/row
 //
 // All FP64 arithmetic on the score path uses explicit round-to-nearest intrinsics in the
@@ -19,7 +19,6 @@
 
 #include <atomic>
 #include <cstdio>
-#include <cstdlib>
 #include <mutex>
 
 namespace tad {
@@ -212,65 +211,6 @@ __global__ void __launch_bounds__(256) partition_kernel(ColPtrs c, uint64_t R, R
                 RowRegs r;
                 load_row_scalar(c, f, i, SCATTER, r);
                 emit_row<SCATTER>(r, bshift, counters, part, opt);
-            }
-        }
-    }
-}
-
-// Scatter, four rows per thread (EXPERIMENT, TAD_SCATTER_RPT=4).  The eight-row kernel above needs 122 registers: two CTAs
-// (16 warps) per SM, and ncu shows it latency bound with head-room everywhere -- 30 of its 35 resident warp-cycles per issued
-// instruction are long-scoreboard waits, L2 at 40 %, DRAM at 27 %, LSU at 31 % (profiles/r01_ncu_full_final.txt).  Half the rows
-// per thread halve the live state: <= 64 registers, four CTAs (32 warps) per SM, twice the loads / atomics / stores in flight.
-__global__ void __launch_bounds__(256, 4) scatter4_kernel(ColPtrs c, uint64_t R, RowFilter f, int bshift,
-                                                          uint32_t *__restrict__ counters, Row32 *__restrict__ part,
-                                                          const OptScatter opt)
-{
-    const uint64_t ngroups = (R + 3) / 4;
-    for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < ngroups; g += (uint64_t)gridDim.x * blockDim.x) {
-        const uint64_t base = g * 4;
-        if (base + 4 <= R) {
-            uint4 z = make_uint4(0, 0, 0, 0);
-            uint4 sip = z, dip = z, fs = z, fe, v0, v1;
-            uint2 sp = make_uint2(0, 0), dp = make_uint2(0, 0);
-            uint32_t pr = 0;
-            if (c.src_ip) sip = ldg_stream128(c.src_ip + base);
-            if (c.dst_ip) dip = ldg_stream128(c.dst_ip + base);
-            if (c.flow_start) fs = ldg_stream128(c.flow_start + base);
-            fe = ldg_stream128(c.flow_end + base);
-            if (c.src_port) sp = ldg_stream64(c.src_port + base);
-            if (c.dst_port) dp = ldg_stream64(c.dst_port + base);
-            if (c.proto) asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(pr) : "l"(c.proto + base));
-            v0 = ldg_stream128(c.value + base);
-            v1 = ldg_stream128(c.value + base + 2);
-            const uint32_t sipv[4] = {sip.x, sip.y, sip.z, sip.w}, dipv[4] = {dip.x, dip.y, dip.z, dip.w};
-            const uint32_t fsv[4] = {fs.x, fs.y, fs.z, fs.w}, fev[4] = {fe.x, fe.y, fe.z, fe.w};
-            const uint32_t spw[2] = {sp.x, sp.y}, dpw[2] = {dp.x, dp.y};
-            const uint32_t vlo[4] = {v0.x, v0.z, v1.x, v1.z}, vhi[4] = {v0.y, v0.w, v1.y, v1.w};
-            RowRegs r[4];
-            uint32_t pos[4], bkt[4];
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const uint32_t sport = (spw[i >> 1] >> (16 * (i & 1))) & 0xffffu;
-                const uint32_t dport = (dpw[i >> 1] >> (16 * (i & 1))) & 0xffffu;
-                r[i].a = pack64(dipv[i], sipv[i]);
-                r[i].b = pack64((sport << 16) | dport, fsv[i]);
-                r[i].proto = (pr >> (8 * i)) & 0xffu;
-                r[i].t = fev[i];
-                r[i].value = pack64(vlo[i], vhi[i]);
-                r[i].keep = row_keep(f, c, base + i, fsv[i], fev[i]);
-                const uint64_t h = key_hash(r[i].a, r[i].b, r[i].proto);
-                bkt[i] = bshift >= 64 ? 0u : (uint32_t)(h >> bshift);
-                r[i].proto |= hash_tag(h, bshift) << 8;
-                pos[i] = r[i].keep ? atomicAdd(&counters[bkt[i]], 1u) : 0xffffffffu;      // four atomics in flight
-            }
-#pragma unroll
-            for (int i = 0; i < 4; i++)
-                if (r[i].keep) place_row(r[i], bkt[i], pos[i], part, opt);
-        } else {
-            for (uint64_t i = base; i < R; i++) {
-                RowRegs r;
-                load_row_scalar(c, f, i, true, r);
-                emit_row<true>(r, bshift, counters, part, opt);
             }
         }
     }
@@ -853,24 +793,6 @@ __device__ __forceinline__ void write_out(const OutCols &o, uint32_t idx, const 
     o.anomaly[idx] = flag ? 1 : 0;
 }
 
-// Visit v[0..n) in order.  `v` points into csr_v (8-byte elements, base 256-byte aligned); after a
-// scalar head the loop reads one full 32-byte sector (four values) per step with two 128-bit loads,
-// so a thread walking its own series never fetches a sector twice.
-template <class F>
-__device__ __forceinline__ void for_each_value(const uint64_t *__restrict__ v, uint32_t n, F &&f)
-{
-    uint32_t i = 0;
-    const uint32_t mis = (uint32_t)((reinterpret_cast<uintptr_t>(v) >> 3) & 3u);
-    const uint32_t head = min(n, (4u - mis) & 3u);
-    for (; i < head; i++) f(v[i], i);
-    for (; i + 4 <= n; i += 4) {
-        const ulonglong2 a = *reinterpret_cast<const ulonglong2 *>(v + i);
-        const ulonglong2 b = *reinterpret_cast<const ulonglong2 *>(v + i + 2);
-        f(a.x, i); f(a.y, i + 1); f(b.x, i + 2); f(b.y, i + 3);
-    }
-    for (; i < n; i++) f(v[i], i);
-}
-
 // Division by the running count on the Welford critical path.  d / k with k a small integer is computed as
 // q0 = d * r (r = RN(1/k) from a table filled with __drcp_rn) plus ONE FMA residual correction
 // q1 = fma(fma(-k, q0, d), r, q0).  That is the correctly rounded quotient: q0 is within 1.5 ulp of z = d/k, so the
@@ -932,136 +854,13 @@ __device__ __forceinline__ double series_stddev(const uint64_t *__restrict__ v, 
     return has_sd ? __dsqrt_rn(__ddiv_rn(m2, __dsub_rn(cnt, 1.0))) : __longlong_as_double(0x7ff8000000000000LL);
 }
 
-// The NT series of a CTA are consecutive in series order, hence (almost always) one contiguous span of
-// csr_v.  The span is staged in shared memory with ONE TMA bulk copy; every thread then runs two sequential
-// passes over its own series out of shared memory (Welford stddev; EWMA + flag).  Flagged points go into a
-// shared-memory queue and are written out cooperatively, one result row per thread, so each of the eleven
-// result columns is written coalesced.  Spans larger than the stage and queue overflows (TAD_FLAG_EMIT_ALL)
-// take the direct per-thread path.
-constexpr int kDetectThreads = 96;
-constexpr int kDetectStage = 10240;                   // staged u64 values per CTA
-constexpr int kDetectQueue = 1024;                    // queued result rows per CTA
-
-template <bool STAGED>
-struct DetectSmem {
-    alignas(128) unsigned long long stage[STAGED ? kDetectStage : 2];
-    double qcalc[kDetectQueue];
-    uint32_t qmeta[kDetectQueue];                     // bit 31: flag, bits 30..16: owning thread, low 16: unused
-    uint32_t qpos[kDetectQueue];                      // index of the point in csr_v / csr_t
-    unsigned long long ent_a[kDetectThreads], ent_b[kDetectThreads];
-    double ent_sd[kDetectThreads];
-    uint32_t ent_proto[kDetectThreads];
-    alignas(8) unsigned long long mbar;
-    uint32_t span_lo, span_hi, qcount, base, b0;
-    uint32_t win[kBucketWindow + 1], woff[kBucketWindow + 1];
-};
-
-template <int NT, bool STAGED>
-__global__ void __launch_bounds__(NT) detect_ewma_kernel(const SeriesEntry *__restrict__ entries, const uint32_t *__restrict__ offsets,
-                                                         const uint32_t *__restrict__ sbase, uint32_t B, uint32_t S,
-                                                         const uint64_t *__restrict__ csr_v, const uint32_t *__restrict__ csr_t,
-                                                         OutCols out, uint32_t out_cap, uint32_t *__restrict__ stats, int emit_all)
-{
-    extern __shared__ __align__(128) unsigned char detect_smem[];
-    DetectSmem<STAGED> &sm = *reinterpret_cast<DetectSmem<STAGED> *>(detect_smem);
-    const uint32_t i = blockIdx.x * NT + threadIdx.x;
-    if (threadIdx.x == 0) {
-        sm.span_lo = 0xffffffffu;
-        sm.span_hi = 0u;
-        sm.qcount = 0u;
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&sm.mbar)), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    SeriesEntry e;
-    e.n = 0; e.off = 0; e.a = 0; e.b = 0; e.proto = 0;
-    const uint32_t bkt = find_bucket_cta(sbase, offsets, B, i < S ? i : S - 1, blockIdx.x * NT, sm.win, sm.woff, &sm.b0);
-    if (i < S) {
-        const uint32_t b = bkt, wk = b - sm.b0;
-        const bool inwin = wk < (uint32_t)kBucketWindow;
-        const uint32_t ob = inwin ? sm.woff[wk] : offsets[b], sb = inwin ? sm.win[wk] : sbase[b];
-        const uint4 *p = reinterpret_cast<const uint4 *>(entries + ob + (i - sb));
-        const uint4 k = p[0], w = p[1];
-        e.a = pack64(k.x, k.y); e.b = pack64(k.z, k.w); e.proto = w.x; e.n = w.y; e.off = w.z;
-    }
-    {
-        const uint32_t lo = __reduce_min_sync(0xffffffffu, e.n ? e.off : 0xffffffffu);
-        const uint32_t hi = __reduce_max_sync(0xffffffffu, e.n ? e.off + e.n : 0u);
-        if ((threadIdx.x & 31) == 0) { atomicMin(&sm.span_lo, lo); atomicMax(&sm.span_hi, hi); }
-    }
-    __syncthreads();
-    const uint32_t lo_a = sm.span_lo & ~3u;                      // keep the 32-byte sector phase of csr_v
-    const bool staged = STAGED && sm.span_hi > lo_a && sm.span_hi - lo_a <= (uint32_t)kDetectStage;
-    if (staged) {
-        if (threadIdx.x == 0) {
-            const uint32_t bytes = ((sm.span_hi - lo_a) * 8u + 15u) & ~15u;
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(&sm.mbar)), "r"(bytes) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         :: "r"(smem_u32(sm.stage)), "l"(csr_v + lo_a), "r"(bytes), "r"(smem_u32(&sm.mbar)) : "memory");
-        }
-        uint32_t done = 0;
-        while (!done) {
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                         : "=r"(done) : "r"(smem_u32(&sm.mbar)), "r"(0) : "memory");
-        }
-    }
-    const uint64_t *v = staged ? reinterpret_cast<const uint64_t *>(sm.stage) + (e.off - lo_a) : csr_v + e.off;
-    bool has_sd = false;
-    double sd = 0.0;
-    if (e.n) {
-        sd = series_stddev(v, e.n, has_sd);
-        sm.ent_a[threadIdx.x] = e.a; sm.ent_b[threadIdx.x] = e.b; sm.ent_proto[threadIdx.x] = e.proto;
-        sm.ent_sd[threadIdx.x] = sd;
-        if (has_sd || emit_all) {
-            double prev = 0.0;
-            for_each_value(v, e.n, [&](uint64_t raw, uint32_t q) {
-                const double x = __ull2double_rn(raw);
-                prev = __dadd_rn(__dmul_rn(0.5, prev), __dmul_rn(0.5, x));
-                const bool flag = has_sd && (fabs(__dsub_rn(x, prev)) > sd);
-                if (flag || emit_all) {
-                    const uint32_t slot = atomicAdd(&sm.qcount, 1u);
-                    if (slot < (uint32_t)kDetectQueue) {
-                        sm.qcalc[slot] = prev;
-                        sm.qpos[slot] = e.off + q;
-                        sm.qmeta[slot] = (flag ? 0x80000000u : 0u) | (threadIdx.x << 16);
-                    } else {                                        // queue full: direct emission
-                        const uint32_t idx = atomicAdd(&stats[ST_OUTCOUNT], 1u);
-                        if (idx < out_cap) write_out(out, idx, e, csr_t[e.off + q], sd, prev, x, flag);
-                    }
-                }
-            });
-        }
-    }
-    __syncthreads();
-    const uint32_t nq = min(sm.qcount, (uint32_t)kDetectQueue);
-    if (threadIdx.x == 0) sm.base = nq ? atomicAdd(&stats[ST_OUTCOUNT], nq) : 0u;
-    __syncthreads();
-    for (uint32_t j = threadIdx.x; j < nq; j += NT) {
-        const uint32_t idx = sm.base + j;
-        if (idx >= out_cap) continue;
-        const uint32_t meta = sm.qmeta[j], pos = sm.qpos[j], owner = (meta >> 16) & 0x7fffu;
-        const uint64_t ka = sm.ent_a[owner], kb = sm.ent_b[owner];
-        out.src_ip[idx] = (uint32_t)(ka >> 32);
-        out.dst_ip[idx] = (uint32_t)ka;
-        out.flow_start[idx] = (uint32_t)(kb >> 32);
-        out.src_port[idx] = (uint16_t)(kb >> 16);
-        out.dst_port[idx] = (uint16_t)kb;
-        out.proto[idx] = (uint8_t)sm.ent_proto[owner];
-        out.flow_end[idx] = csr_t[pos];
-        out.stddev[idx] = sm.ent_sd[owner];
-        out.algo_calc[idx] = sm.qcalc[j];
-        out.throughput[idx] = __ull2double_rn(staged ? sm.stage[pos - lo_a] : csr_v[pos]);
-        out.anomaly[idx] = (meta >> 31) ? 1 : 0;
-    }
-}
-
 // ----------------------------------------------------------------------------------------
-// K4, direct variant: no shared-memory stage.  A thread streams its own series straight out of csr_v, one full
+// K4 (EWMA): no shared-memory stage.  A thread streams its own series straight out of csr_v, one full
 // 32-byte sector (four values, ONE 256-bit load through the read-only path) per step with the next sector already
 // in flight, so no sector is fetched twice and the kernel runs at register-limited occupancy (5 CTAs of 128 threads
-// per SM instead of two of 96).  The staged variant is latency bound -- 6 warps per SM on dependent FP64 chains issue
-// ~0.75 instructions per clock and SM (profiles/r01_source_lines_detect.txt) -- and this one attacks exactly that with
-// more warps.  Sectors are addressed from the sector-aligned start of the series (csr_v is padded by one sector),
+// per SM instead of two of 96).  The round-1 detector staged each CTA's span in shared memory with TMA and was latency
+// bound -- 6 warps per SM on dependent FP64 chains issue ~0.75 instructions per clock and SM
+// (profiles/r01_source_lines_detect.txt) -- and this one attacks exactly that with more warps.  Sectors are addressed from the sector-aligned start of the series (csr_v is padded by one sector),
 // elements outside [0, n) are masked.  Flagged points are queued in shared memory (one warp-aggregated atomic per
 // flagged point) and written out cooperatively, every result column coalesced.
 // ----------------------------------------------------------------------------------------
@@ -1389,17 +1188,7 @@ cudaError_t launch_scatter(cudaStream_t st, const ColPtrs &c, uint64_t R, const 
     if (R == 0) return cudaSuccess;
     const int bshift = 64 - logB;
     const OptScatter opt{slot_cap, ovf_cap, ovf, ovf_count};
-    static std::atomic<int> rpt_s{0};
-    int rpt = rpt_s.load(std::memory_order_relaxed);
-    if (!rpt) {
-        const char *ev = getenv("TAD_SCATTER_RPT");           // rows per thread of the scatter: 8 (122 registers) or 4 (<= 64)
-        rpt = ev && atoi(ev) == 4 ? 4 : 8;
-        rpt_s.store(rpt, std::memory_order_relaxed);
-    }
-    if (rpt == 4 && cols_aligned16(c) && c.flow_end && c.value) {
-        const uint64_t want = ((R + 3) / 4 + 255) / 256, cap = (uint64_t)num_sms() * 4 * 4;
-        scatter4_kernel<<<(uint32_t)(want < cap ? (want ? want : 1) : cap), 256, 0, st>>>(c, R, f, bshift, cursor, part, opt);
-    } else if (cols_aligned16(c))
+    if (cols_aligned16(c))
         partition_kernel<true, true><<<partition_grid(R), 256, 0, st>>>(c, R, f, bshift, cursor, part, opt);
     else
         partition_kernel<true, false><<<partition_grid(R), 256, 0, st>>>(c, R, f, bshift, cursor, part, opt);
@@ -1449,63 +1238,37 @@ static cudaError_t launch_group_class(cudaStream_t st, const SegDesc &seg, Serie
 // listed bucket -- launching all B CTAs per class and exiting early costs ~0.5 ms per class at 180 KB of shared
 // memory per CTA.  Empty buckets keep the zeroes the caller memset into nsb / npb.
 template <bool VRANK>
-static cudaError_t launch_group_all(cudaStream_t st, const GroupStreams *gs, const SegDesc &seg, SeriesEntry *entries,
-                                    const uint32_t *offsets, uint32_t B, const uint32_t *cls_list, const uint32_t n_cls[3],
-                                    uint64_t *csr_v, uint32_t *csr_t, uint32_t *csr_p, uint32_t *nsb, uint32_t *npb, int reducer,
-                                    int *launches)
+static cudaError_t launch_group_all(cudaStream_t st, const SegDesc &seg, SeriesEntry *entries, const uint32_t *offsets,
+                                    uint32_t B, const uint32_t *cls_list, const uint32_t n_cls[3], uint64_t *csr_v,
+                                    uint32_t *csr_t, uint32_t *csr_p, uint32_t *nsb, uint32_t *npb, int reducer, int *launches)
 {
-    static std::atomic<int> small_nt_s{0};
-    int small_nt = small_nt_s.load(std::memory_order_relaxed);
-    if (!small_nt) {
-        const char *ev = getenv("TAD_GROUP_NT");          // tuning knob: threads per CTA of the first capacity class
-        small_nt = ev ? atoi(ev) : 256;
-        small_nt_s.store(small_nt, std::memory_order_relaxed);
-    }
     *launches = 0;
-    // The three classes work on disjoint buckets.  With `gs` the two large classes (one or two CTAs per SM by shared memory)
-    // run on side streams NEXT TO the first class instead of after it: their few big CTAs start first, the small CTAs fill
-    // the rest of every SM, and the low-occupancy tails of the three launches overlap.
-    cudaStream_t s1 = st, s2 = st;
-    const bool fork = gs != nullptr && (n_cls[1] || n_cls[2]);
     cudaError_t e = cudaSuccess;
-    if (fork) {
-        e = cudaEventRecord(gs->fork, st);
-        if (e == cudaSuccess && n_cls[1]) { s1 = gs->aux[0]; e = cudaStreamWaitEvent(s1, gs->fork, 0); }
-        if (e == cudaSuccess && n_cls[2]) { s2 = gs->aux[1]; e = cudaStreamWaitEvent(s2, gs->fork, 0); }
-    }
-    if (e == cudaSuccess && n_cls[2]) {
-        e = launch_group_class<kGroupCap, 512, VRANK>(s2, seg, entries, offsets, cls_list + 2 * (size_t)B, n_cls[2], kGroupCapMid,
+    if (n_cls[2]) {
+        e = launch_group_class<kGroupCap, 512, VRANK>(st, seg, entries, offsets, cls_list + 2 * (size_t)B, n_cls[2], kGroupCapMid,
                                                       csr_v, csr_t, csr_p, nsb, npb, reducer);
         ++*launches;
     }
     if (e == cudaSuccess && n_cls[1]) {
-        e = launch_group_class<kGroupCapMid, 256, VRANK>(s1, seg, entries, offsets, cls_list + B, n_cls[1], kGroupCapSmall,
+        e = launch_group_class<kGroupCapMid, 256, VRANK>(st, seg, entries, offsets, cls_list + B, n_cls[1], kGroupCapSmall,
                                                          csr_v, csr_t, csr_p, nsb, npb, reducer);
         ++*launches;
     }
     if (e == cudaSuccess) {
-        e = small_nt == 128
-                ? launch_group_class<kGroupCapSmall, 128, VRANK>(st, seg, entries, offsets, cls_list, n_cls[0], 0, csr_v, csr_t,
-                                                                 csr_p, nsb, npb, reducer)
-                : launch_group_class<kGroupCapSmall, 256, VRANK>(st, seg, entries, offsets, cls_list, n_cls[0], 0, csr_v, csr_t,
-                                                                 csr_p, nsb, npb, reducer);
+        e = launch_group_class<kGroupCapSmall, 256, VRANK>(st, seg, entries, offsets, cls_list, n_cls[0], 0, csr_v, csr_t,
+                                                           csr_p, nsb, npb, reducer);
         *launches += n_cls[0] ? 1 : 0;
-    }
-    if (fork) {          // join: the main stream continues when all classes are done (also after an error above)
-        if (n_cls[1]) { cudaEventRecord(gs->join[0], s1); cudaStreamWaitEvent(st, gs->join[0], 0); }
-        if (n_cls[2]) { cudaEventRecord(gs->join[1], s2); cudaStreamWaitEvent(st, gs->join[1], 0); }
     }
     return e;
 }
 
 cudaError_t launch_group(cudaStream_t st, const SegDesc &seg, SeriesEntry *entries, const uint32_t *offsets, uint32_t B,
-                         int logB, const uint32_t *cls_list, const uint32_t n_cls[3], uint64_t *csr_v, uint32_t *csr_t,
-                         uint32_t *csr_p, uint32_t *nsb, uint32_t *npb, int reducer, int *launches, const GroupStreams *gs)
+                         const uint32_t *cls_list, const uint32_t n_cls[3], uint64_t *csr_v, uint32_t *csr_t,
+                         uint32_t *csr_p, uint32_t *nsb, uint32_t *npb, int reducer, int *launches)
 {
-    (void)logB;        // the slot hash bits travel with the rows (hash_tag)
-    return csr_p ? launch_group_all<true>(st, gs, seg, entries, offsets, B, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb,
+    return csr_p ? launch_group_all<true>(st, seg, entries, offsets, B, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb,
                                           reducer, launches)
-                 : launch_group_all<false>(st, gs, seg, entries, offsets, B, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb,
+                 : launch_group_all<false>(st, seg, entries, offsets, B, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb,
                                            reducer, launches);
 }
 
@@ -1530,36 +1293,9 @@ cudaError_t launch_detect_ewma(cudaStream_t st, const SeriesEntry *entries, cons
                                uint32_t out_cap, uint32_t *stats, int emit_all)
 {
     if (S == 0) return cudaSuccess;
-    constexpr int NT = kDetectThreads;
-    static std::atomic<int> staged_s{-1};
-    int staged = staged_s.load(std::memory_order_acquire);
-    if (staged < 0) {
-        const char *ev = getenv("TAD_DETECT_STAGED");        // tuning knob: 1 = TMA-staged span (2 CTAs/SM), 0 = global loads at full occupancy
-        staged = ev ? atoi(ev) : 1;
-        cudaError_t e = cudaFuncSetAttribute(detect_ewma_kernel<NT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)sizeof(DetectSmem<true>));
-        if (e != cudaSuccess) return e;
-        staged_s.store(staged, std::memory_order_release);
-    }
     ensure_rcp_table(st);
-    static std::atomic<int> mode_s{-1};
-    int mode = mode_s.load(std::memory_order_acquire);
-    if (mode < 0) {
-        const char *ev = getenv("TAD_DETECT_MODE");          // 1 = direct (no stage, register-limited occupancy; 0.63 vs 1.10 ms
-        mode = ev ? atoi(ev) : 1;                            // per 1e8 points, profiles/r02/ab2_summary.txt), 0 = TMA-staged
-        mode_s.store(mode, std::memory_order_release);
-    }
-    if (mode == 1) {
-        detect_ewma_direct_kernel<kDirectThreads><<<(S + kDirectThreads - 1) / kDirectThreads, kDirectThreads, 0, st>>>(
-            entries, offsets, sbase, B, S, csr_v, csr_t, out, out_cap, stats, emit_all);
-        return cudaGetLastError();
-    }
-    if (staged)
-        detect_ewma_kernel<NT, true><<<(S + NT - 1) / NT, NT, sizeof(DetectSmem<true>), st>>>(entries, offsets, sbase, B, S, csr_v, csr_t,
-                                                                                            out, out_cap, stats, emit_all);
-    else
-        detect_ewma_kernel<NT, false><<<(S + NT - 1) / NT, NT, sizeof(DetectSmem<false>), st>>>(entries, offsets, sbase, B, S, csr_v,
-                                                                                              csr_t, out, out_cap, stats, emit_all);
+    detect_ewma_direct_kernel<kDirectThreads><<<(S + kDirectThreads - 1) / kDirectThreads, kDirectThreads, 0, st>>>(
+        entries, offsets, sbase, B, S, csr_v, csr_t, out, out_cap, stats, emit_all);
     return cudaGetLastError();
 }
 

@@ -1,4 +1,4 @@
-// Launchers of the TAD engine kernels (implemented in tad_kernels.cu, tad_spill.cu, tad_dbscan.cu).
+// Launchers of the TAD engine kernels (implemented in tad_kernels.cu, tad_spill.cu, tad_arima.cu).
 #pragma once
 #include "tad_common.cuh"
 
@@ -19,15 +19,9 @@ size_t scan_sync_bytes();   // zero-initialised once; epoch must be > 0 and diff
 // index) the DBSCAN detector sweeps over.
 // `offsets` are the (virtual, contiguous) bucket offsets used for entries / csr arrays; the rows
 // themselves are read through `seg`.
-// gs != nullptr: the capacity classes run concurrently (two side streams, fork / join events owned by the caller).
-struct GroupStreams {
-    cudaStream_t aux[2];
-    cudaEvent_t fork, join[2];
-};
 cudaError_t launch_group(cudaStream_t st, const SegDesc &seg, SeriesEntry *entries, const uint32_t *offsets, uint32_t B,
-                         int logB, const uint32_t *cls_list, const uint32_t n_cls[3], uint64_t *csr_v, uint32_t *csr_t,
-                         uint32_t *csr_p, uint32_t *nsb, uint32_t *npb, int reducer, int *launches,
-                         const GroupStreams *gs = nullptr);
+                         const uint32_t *cls_list, const uint32_t n_cls[3], uint64_t *csr_v, uint32_t *csr_t,
+                         uint32_t *csr_p, uint32_t *nsb, uint32_t *npb, int reducer, int *launches);
 cudaError_t launch_series_scan(cudaStream_t st, const uint32_t *nsb, const uint32_t *npb, uint32_t *sbase, uint32_t B,
                                uint32_t *stats, void *scan_sync, uint32_t epoch);
 cudaError_t launch_detect_ewma(cudaStream_t st, const SeriesEntry *entries, const uint32_t *offsets, const uint32_t *sbase, uint32_t B,
