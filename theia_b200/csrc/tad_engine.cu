@@ -26,9 +26,13 @@ using namespace tad;
 
 namespace {
 
-struct DevBuf {
+struct DevBuf {            // grow-only device buffer (ensure()); freed with the context that owns it
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;               // owns its allocation
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
 };
 
 struct PinnedBlock {
@@ -41,6 +45,24 @@ constexpr int kMaxChunks = 16;          // host-resident input is copied and his
 constexpr int kMaxRanks = 8;
 constexpr int kMaxXChunks = kMaxSeg / kMaxRanks;   // exchange chunks: scatter of chunk c+1 overlaps the all-to-all of chunk c
 constexpr int kTotalStages = 6;   // ingest, partition, exchange, group, detect, egress
+
+// Layout of the scratch words (u64) of `small` (device, 4096 bytes) and `h_small` (pinned, kSmallWords).  An all-gather
+// sends from one slot and receives one entry per rank at another.  Each slot names the phase that owns it.
+enum SmallSlot : int {
+    kSlotSend = 0,            // agree on rows, gather16: this rank's entry of the all-gather
+    kSlotSegRows = 0,         // exact multi-GPU partition: rows of each (source rank, chunk) segment in the owned range
+    kSlotRows = 8,            // agree on rows: every rank's row count
+    kSlotGather16 = 16,       // gather16 (exported-buffer handles, largest shard): 16 words per rank
+    kSlotOvf = 32,            // optimistic peer pull: every rank's overflow count
+    kSlotFront = 40,          // exact peer pull: rows in front of the owned range in each source's partition
+    kSlotBarrier = 48,        // barrier(): the word every rank sends
+    kSlotBarrierRecv = 56,    // barrier(): the words every rank receives
+    kSlotSendLo = 64,         // exact multi-GPU partition (host only): kMaxRanks + 1 send boundaries per exchange chunk
+    kSmallWords = 256,
+};
+static_assert(kSlotSegRows + kMaxSeg <= kSlotFront, "segment rows and the rows in front of the owned range overlap");
+static_assert(kSlotFront + kMaxRanks <= kSlotBarrier, "the rows in front of the owned range overlap the barrier");
+static_assert(kSlotSendLo + kMaxXChunks * (kMaxRanks + 1) <= kSmallWords, "send boundaries overrun h_small");
 
 // ---- NUMA placement of pinned host memory --------------------------------------------------------------------------
 // On a two-socket box half of the GPUs hang off each socket; a pinned buffer on the wrong socket makes every H2D / D2H
@@ -164,12 +186,11 @@ struct tad_ctx {
     bool stop = false;
     int debug_logb = -1;
     int debug_target = 0;      // TAD_GROUP_TARGET: mean rows per bucket (tuning)
-    int num_sms = 148;
     // device workspace (grow-only, reused across jobs; jobs are serialized by the worker)
     DevBuf d_col[10], hist, offsets, cursor, big_list, big_base, cls_list, csr_p, stats, part, csr_v, csr_t, nsb, npb, sbase, outb, ns_ignore, spill,
         dbx, dbi, exch, scan_sync, small, hist_all, seg_off, seg_total, entries, ar_y, ar_pred, ar_lam, ovf;
     int optimistic = 1;      // TAD_OPTIMISTIC=0: always the exact (histogram + scan + scatter) partition
-    unsigned long long *h_small = nullptr;   // pinned, 256 x u64
+    unsigned long long *h_small = nullptr;   // pinned, kSmallWords x u64 (layout: SmallSlot)
     uint32_t scan_epoch = 0;
     uint32_t *h_stats = nullptr;   // pinned readback of the device scalars
     std::mutex pool_mu;
@@ -219,9 +240,9 @@ struct JobFail {
                  cudaGetErrorString(_e), __FILE__, __LINE__);                                            \
     } while (0)
 
-void ensure(DevBuf &b, size_t bytes)
+void *ensure(DevBuf &b, size_t bytes)      // returns b.p
 {
-    if (bytes <= b.cap) return;
+    if (bytes <= b.cap) return b.p;
     if (b.p) CU(cudaFree(b.p));
     b.p = nullptr;
     b.cap = 0;
@@ -234,6 +255,7 @@ void ensure(DevBuf &b, size_t bytes)
         CU(cudaMalloc(&b.p, want));
     }
     b.cap = want;
+    return b.p;
 }
 
 PinnedBlock take_pinned(tad_ctx *ctx, size_t bytes)
@@ -346,221 +368,241 @@ OutCols out_cols(void *base, const OutLayout &L)
     return o;
 }
 
-void run_job(tad_ctx *ctx, tad_job *job)
-{
-    const tad_job_spec &sp = job->spec;
-    const tad_columns &hc = job->cols;
-    const uint64_t R = hc.rows;
-    cudaStream_t st = ctx->stream;
-    uint64_t launches = 0;
-    int nev = 0;
-    int ev_phase[kMaxEvents];
-    auto mark = [&](int phase) {          // event closing `phase`
-        if (nev < kMaxEvents) {
-            CU(cudaEventRecord(ctx->ev[nev], st));
-            ev_phase[nev++] = phase;
-        }
-    };
-    auto check_cancel = [&]() {
-        if (job->cancel.load()) fail(TAD_ERR_CANCELLED, "job cancelled");
-    };
+void nccl_ok(int rc) { if (rc) fail(TAD_ERR_NCCL, "%s", nccl_last_error()); }
 
-    CU(cudaSetDevice(ctx->cfg.device));
-    set_progress(job, TAD_STATE_RUNNING, 0);
-    ensure(ctx->stats, 64 * sizeof(uint32_t));
-    uint32_t *d_stats = static_cast<uint32_t *>(ctx->stats.p);
-    CU(cudaMemsetAsync(d_stats, 0, 64 * sizeof(uint32_t), st));
-    if (!ctx->scan_sync.p) {
-        ensure(ctx->scan_sync, scan_sync_bytes());
-        CU(cudaMemsetAsync(ctx->scan_sync.p, 0, scan_sync_bytes(), st));
+// Barrier of all ranks on the job stream (an 8-byte all-gather).  Returns the NCCL status.
+int barrier(tad_ctx *ctx)
+{
+    unsigned long long *d = static_cast<unsigned long long *>(ctx->small.p);
+    return nccl_allgather(&ctx->nccl, d + kSlotBarrier, d + kSlotBarrierRecv, 8, ctx->stream);
+}
+
+// What a partition path leaves for the group phase: where the rows of each owned bucket are, and the row counts.
+struct Partition {
+    SegDesc seg{};
+    SeriesEntry *entries = nullptr;
+    uint64_t kept = 0, owned = 0;          // rows of this rank that passed the filters / rows of its bucket range
+    const Row32 *ovf_rows = nullptr;       // single-GPU optimistic partition: rows that found their slot full
+    uint32_t n_ovf = 0;
+    bool sync_at_end = false;              // peers read this rank's exported rows: meet them before the next job
+};
+
+// One job on the worker thread.  run_job calls the phases in order; the members are what the phases share.
+struct JobRun {
+    tad_ctx *const ctx;
+    tad_job *const job;
+    const tad_job_spec &sp;
+    const cudaStream_t st;
+    const uint64_t R;                      // rows of this rank
+    const bool host_input;
+    const int world, me;
+    int nchunks = 1;                       // H2D chunks of host input
+    const void *dcol[10]{};                // device columns (the caller's own when device-resident)
+    ColPtrs c{};
+    RowFilter f{};
+    uint32_t *d_stats = nullptr;
+    unsigned long long *d_small = nullptr;     // layout: SmallSlot
+    uint64_t R_total = 0;                  // rows of all ranks
+    int logB = 0;                          // B global buckets; this rank owns the Bl buckets from b_lo on
+    uint32_t B = 0, Bl = 0, b_lo = 0;
+    uint32_t slotM = 0;                    // multi-GPU optimistic partition: slot rows per (bucket, source rank)
+    size_t x_cnt_bytes = 0;                // exported buffer: arrival counters in front of the rows
+    uint32_t *hist = nullptr, *offsets = nullptr, *cursor = nullptr, *big_list = nullptr, *big_base = nullptr;
+    uint32_t *cls_list = nullptr, *nsb = nullptr, *npb = nullptr;
+    uint64_t *csr_v = nullptr;             // grouped series (CSR) and series base per bucket
+    uint32_t *csr_t = nullptr, *csr_p = nullptr, *sbase = nullptr;
+    uint64_t launches = 0;
+    int nev = 0, ev_phase[kMaxEvents];
+
+    JobRun(tad_ctx *ctx_, tad_job *job_)
+        : ctx(ctx_), job(job_), sp(job_->spec), st(ctx_->stream), R(job_->cols.rows),
+          host_input(job_->cols.mem != TAD_MEM_DEVICE && R > 0), world(ctx_->cfg.world_size), me(ctx_->cfg.rank) {}
+    // event closing `phase`
+    void mark(int phase) { if (nev < kMaxEvents) { CU(cudaEventRecord(ctx->ev[nev], st)); ev_phase[nev++] = phase; } }
+    void check_cancel() { if (job->cancel.load()) fail(TAD_ERR_CANCELLED, "job cancelled"); }
+    void read_stats()             // device scalars -> ctx->h_stats
+    {
+        CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    void allgather(const void *send, void *recv, size_t bytes) { nccl_ok(nccl_allgather(&ctx->nccl, send, recv, bytes, st)); }
+    SeriesEntry *use_entries(uint64_t owned) { return (SeriesEntry *)ensure(ctx->entries, (owned ? owned : 1) * sizeof(SeriesEntry)); }
+    const Row32 *peer_rows(int r) const      // the rows of rank r's exported buffer (this rank's own for r == me)
+    {
+        return reinterpret_cast<const Row32 *>(static_cast<const char *>(r == me ? ctx->xbuf.p : ctx->peer_x[r]) + x_cnt_bytes);
+    }
+    uint64_t split(int k, int n) const       // first row of piece k of n (k = n: R); keeps every column 16-byte aligned
+    {
+        if (k <= 0 || k >= n) return k <= 0 ? 0 : R;
+        const uint64_t v = ((R * (uint64_t)k / n) + 15) & ~uint64_t(15);
+        return v < R ? v : R;
+    }
+    ColPtrs offset_cols(uint64_t lo) const   // the device columns from row lo on
+    {
+        auto at = [&](int i) { return dcol[i] ? static_cast<const char *>(dcol[i]) + col_bytes(i, lo) : nullptr; };
+        ColPtrs ck;
+        ck.src_ip = (const uint32_t *)at(0); ck.dst_ip = (const uint32_t *)at(1);
+        ck.src_port = (const uint16_t *)at(2); ck.dst_port = (const uint16_t *)at(3);
+        ck.proto = (const uint8_t *)at(4); ck.flow_start = (const uint32_t *)at(5);
+        ck.flow_end = (const uint32_t *)at(6); ck.value = (const uint64_t *)at(7);
+        ck.src_ns = (const uint32_t *)at(8); ck.dst_ns = (const uint32_t *)at(9);
+        return ck;
+    }
+    // First pass over the input: launch(cols, rows) on each H2D chunk once it has landed (host input; the copy and the
+    // overlapped pass are accounted as TAD_PHASE_H2D), or once on the device-resident columns.
+    template <class Launch>
+    void over_input(int phase_if_device, Launch launch)
+    {
+        if (host_input) {
+            for (int k = 0; k < nchunks; k++) {
+                const uint64_t lo = split(k, nchunks), hi = split(k + 1, nchunks);
+                CU(cudaStreamWaitEvent(st, ctx->chunk_ev[k], 0));
+                if (hi <= lo) continue;
+                CU(launch(offset_cols(lo), hi - lo)); launches++;
+            }
+            mark(TAD_PHASE_H2D);
+        } else {
+            CU(launch(c, R)); launches += R ? 1 : 0;
+            mark(phase_if_device);
+        }
     }
 
     // ---- ingest: host columns -> device (device-resident columns are used in place) -------
     // Host input is copied in chunks on a second stream; the bucket histogram is additive, so the
     // histogram of chunk i runs while chunk i+1 is still on the PCIe bus.
-    ColPtrs c{};
-    const void *dcol[10];
-    const bool host_input = hc.mem != TAD_MEM_DEVICE && R > 0;
-    for (int i = 0; i < 10; i++) {
-        void *src = col_ptr(hc, i);
-        dcol[i] = nullptr;
-        if (!src || R == 0) continue;
-        if (hc.mem == TAD_MEM_DEVICE) {
-            dcol[i] = src;
-        } else {
-            ensure(ctx->d_col[i], col_bytes(i, R));
-            dcol[i] = ctx->d_col[i].p;
+    void ingest()
+    {
+        CU(cudaSetDevice(ctx->cfg.device));
+        set_progress(job, TAD_STATE_RUNNING, 0);
+        d_stats = (uint32_t *)ensure(ctx->stats, 64 * sizeof(uint32_t));
+        CU(cudaMemsetAsync(d_stats, 0, 64 * sizeof(uint32_t), st));
+        if (!ctx->scan_sync.p) CU(cudaMemsetAsync(ensure(ctx->scan_sync, scan_sync_bytes()), 0, scan_sync_bytes(), st));
+        const tad_columns &hc = job->cols;
+        for (int i = 0; i < 10; i++) {
+            void *src = col_ptr(hc, i);
+            if (src && R > 0) dcol[i] = hc.mem == TAD_MEM_DEVICE ? src : ensure(ctx->d_col[i], col_bytes(i, R));
         }
-    }
-    int nchunks = 1;
-    if (host_input) {
-        nchunks = (int)((R + (8u << 20) - 1) / (8u << 20));          // ~8M rows (232 MB) per chunk
-        if (nchunks > kMaxChunks) nchunks = kMaxChunks;
-        if (nchunks < 1) nchunks = 1;
-    }
-    auto chunk_lo = [&](int k) { return ((R * (uint64_t)k / nchunks) + 15) & ~uint64_t(15); };   // keeps every column 16-byte aligned
-    auto chunk_range = [&](int k, uint64_t &lo, uint64_t &hi) {
-        lo = k == 0 ? 0 : (chunk_lo(k) < R ? chunk_lo(k) : R);
-        hi = k + 1 == nchunks ? R : (chunk_lo(k + 1) < R ? chunk_lo(k + 1) : R);
-    };
-    mark(-1);
-    if (host_input) {
-        CU(cudaEventRecord(ctx->start_ev, st));
-        CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->start_ev, 0));   // workspace of the previous job is free
-        for (int k = 0; k < nchunks; k++) {
-            uint64_t lo, hi;
-            chunk_range(k, lo, hi);
-            for (int i = 0; i < 10 && hi > lo; i++) {
-                const char *src = static_cast<const char *>(col_ptr(hc, i));
-                if (!src) continue;
-                const size_t w = col_bytes(i, 1);
-                CU(cudaMemcpyAsync(static_cast<char *>(ctx->d_col[i].p) + lo * w, src + lo * w, (hi - lo) * w,
-                                   cudaMemcpyHostToDevice, ctx->copy_stream));
+        if (host_input)            // ~8M rows (232 MB) per chunk
+            nchunks = (int)std::min<uint64_t>(kMaxChunks, (R + (8u << 20) - 1) / (8u << 20));
+        mark(-1);
+        if (host_input) {
+            CU(cudaEventRecord(ctx->start_ev, st));
+            CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->start_ev, 0));   // workspace of the previous job is free
+            for (int k = 0; k < nchunks; k++) {
+                const uint64_t lo = split(k, nchunks), hi = split(k + 1, nchunks);
+                for (int i = 0; i < 10 && hi > lo; i++)
+                    if (dcol[i])
+                        CU(cudaMemcpyAsync((char *)dcol[i] + col_bytes(i, lo), (const char *)col_ptr(hc, i) + col_bytes(i, lo),
+                                           col_bytes(i, hi - lo), cudaMemcpyHostToDevice, ctx->copy_stream));
+                CU(cudaEventRecord(ctx->chunk_ev[k], ctx->copy_stream));
             }
-            CU(cudaEventRecord(ctx->chunk_ev[k], ctx->copy_stream));
+        }
+        c = offset_cols(0);
+        f.start_time = sp.start_time; f.end_time = sp.end_time;
+        if (!job->ns_ignore.empty() && (c.src_ns || c.dst_ns)) {
+            ensure(ctx->ns_ignore, job->ns_ignore.size() * 4);
+            CU(cudaMemcpyAsync(ctx->ns_ignore.p, job->ns_ignore.data(), job->ns_ignore.size() * 4, cudaMemcpyHostToDevice, st));
+            f.n_ns_ignore = (uint32_t)job->ns_ignore.size();
+            f.ns_ignore = static_cast<const uint32_t *>(ctx->ns_ignore.p);
         }
     }
-    c.src_ip = (const uint32_t *)dcol[0]; c.dst_ip = (const uint32_t *)dcol[1];
-    c.src_port = (const uint16_t *)dcol[2]; c.dst_port = (const uint16_t *)dcol[3];
-    c.proto = (const uint8_t *)dcol[4]; c.flow_start = (const uint32_t *)dcol[5];
-    c.flow_end = (const uint32_t *)dcol[6]; c.value = (const uint64_t *)dcol[7];
-    c.src_ns = (const uint32_t *)dcol[8]; c.dst_ns = (const uint32_t *)dcol[9];
-
-    RowFilter f{};
-    f.start_time = sp.start_time;
-    f.end_time = sp.end_time;
-    if (!job->ns_ignore.empty() && (c.src_ns || c.dst_ns)) {
-        ensure(ctx->ns_ignore, job->ns_ignore.size() * 4);
-        CU(cudaMemcpyAsync(ctx->ns_ignore.p, job->ns_ignore.data(), job->ns_ignore.size() * 4, cudaMemcpyHostToDevice, st));
-        f.n_ns_ignore = (uint32_t)job->ns_ignore.size();
-        f.ns_ignore = static_cast<const uint32_t *>(ctx->ns_ignore.p);
+    // ---- agree on the rows of the table, pick the buckets (the same global count on every rank) ----------------------
+    void pick_buckets()
+    {
+        R_total = R;
+        d_small = (unsigned long long *)ensure(ctx->small, 4096);
+        if (world > 1 && sp.global_rows) {
+            R_total = sp.global_rows;      // the host counted the table: no start-of-job collective, no host sync
+        } else if (world > 1) {
+            ctx->h_small[kSlotSend] = R;
+            CU(cudaMemcpyAsync(d_small + kSlotSend, ctx->h_small + kSlotSend, 8, cudaMemcpyHostToDevice, st));
+            allgather(d_small + kSlotSend, d_small + kSlotRows, 8);
+            CU(cudaMemcpyAsync(ctx->h_small, d_small + kSlotRows, 8 * world, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            mark(TAD_PHASE_SYNC);          // arrival skew of the ranks at job start (avoided when the host passes global_rows)
+            R_total = 0;
+            for (int r = 0; r < world; r++) R_total += ctx->h_small[r];
+        }
+        logB = pick_logb(ctx, R_total);
+        int logW = 0;
+        while ((1 << logW) < world) logW++;
+        if (logB < logW) logB = logW;
+        B = 1u << logB;                 // global buckets
+        Bl = B >> logW;                 // buckets owned by one rank
+        b_lo = Bl * (uint32_t)me;
+        slotM = std::max<uint32_t>(256u, (uint32_t)kGroupCap / (uint32_t)world);
+        x_cnt_bytes = (((size_t)B * 4) + 65535) & ~size_t(65535);
+        hist = (uint32_t *)ensure(ctx->hist, (size_t)B * 4);
+        offsets = (uint32_t *)ensure(ctx->offsets, ((size_t)B + 1) * 4);
+        cursor = (uint32_t *)ensure(ctx->cursor, (size_t)B * 4);
+        big_list = (uint32_t *)ensure(ctx->big_list, (size_t)B * 4);
+        big_base = (uint32_t *)ensure(ctx->big_base, ((size_t)B + 1) * 4);
+        cls_list = (uint32_t *)ensure(ctx->cls_list, (size_t)B * 4 * 3);
+        nsb = (uint32_t *)ensure(ctx->nsb, (size_t)Bl * 4);
+        npb = (uint32_t *)ensure(ctx->npb, (size_t)Bl * 4);
+        // part[] (exact partition: 32 B per local row) is not needed when the multi-GPU optimistic path runs out of the exported
+        // slot buffer; the exact multi-GPU branch allocates it on demand
+        if (world == 1) ensure(ctx->part, (R ? R : 1) * sizeof(Row32));
+        CU(cudaMemsetAsync(nsb, 0, (size_t)Bl * 4, st));
+        CU(cudaMemsetAsync(npb, 0, (size_t)Bl * 4, st));
     }
-
-    // ---- partition -------------------------------------------------------------------------
-    const int world = ctx->cfg.world_size, me = ctx->cfg.rank;
-    uint64_t R_total = R;
-    ensure(ctx->small, 4096);
-    unsigned long long *d_small = static_cast<unsigned long long *>(ctx->small.p);
-    if (world > 1 && sp.global_rows) {
-        R_total = sp.global_rows;      // the host counted the table: no start-of-job collective, no host sync
-    } else if (world > 1) {
-        // global row count -> same bucket count on every rank
-        ctx->h_small[0] = R;
-        CU(cudaMemcpyAsync(d_small, ctx->h_small, 8, cudaMemcpyHostToDevice, st));
-        if (nccl_allgather(&ctx->nccl, d_small, d_small + 8, 8, st)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
-        CU(cudaMemcpyAsync(ctx->h_small, d_small + 8, 8 * world, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        mark(TAD_PHASE_SYNC);          // arrival skew of the ranks at job start (avoided when the host passes global_rows)
-        R_total = 0;
-        for (int r = 0; r < world; r++) R_total += ctx->h_small[r];
+    // ---- partition: an optimistic path where it applies; where it falls back, the exact path for the world size
+    Partition partition()
+    {
+        Partition p;
+        if (world == 1 && ctx->optimistic && R > 0 && (uint64_t)B * kGroupCap * sizeof(Row32) <= (64ull << 30) &&
+            local_slots(p))
+            return p;
+        const size_t x_need = x_cnt_bytes + (size_t)B * slotM * sizeof(Row32);
+        if (world > 1 && ctx->peer_pull && ctx->optimistic && R_total > 0 && (uint64_t)B * slotM <= (1ull << 31) &&
+            x_need <= ctx->x_budget && peer_slots(p, x_need))
+            return p;
+        return world == 1 ? exact_local() : exact_multi();
     }
-    int logB = pick_logb(ctx, R_total);
-    int logW = 0;
-    while ((1 << logW) < world) logW++;
-    if (logB < logW) logB = logW;
-    const uint32_t B = 1u << logB;                 // global buckets
-    const uint32_t Bl = B >> logW;                 // buckets owned by one rank
-    const uint32_t b_lo = Bl * (uint32_t)me;
-    ensure(ctx->hist, (size_t)B * 4);
-    ensure(ctx->offsets, ((size_t)B + 1) * 4);
-    ensure(ctx->cursor, (size_t)B * 4);
-    ensure(ctx->big_list, (size_t)B * 4);
-    ensure(ctx->big_base, ((size_t)B + 1) * 4);
-    ensure(ctx->cls_list, (size_t)B * 4 * 3);
-    ensure(ctx->nsb, (size_t)Bl * 4);
-    ensure(ctx->npb, (size_t)Bl * 4);
-    // part[] (exact partition: 32 B per local row) is not needed when the multi-GPU optimistic path runs out of the exported
-    // slot buffer; the exact multi-GPU branch allocates it on demand
-    if (world == 1) ensure(ctx->part, (R ? R : 1) * sizeof(Row32));
-    uint32_t *hist = (uint32_t *)ctx->hist.p, *offsets = (uint32_t *)ctx->offsets.p, *cursor = (uint32_t *)ctx->cursor.p;
-    uint32_t *big_base = (uint32_t *)ctx->big_base.p;
-    uint32_t *cls_list = (uint32_t *)ctx->cls_list.p;
-    uint32_t *big_list = (uint32_t *)ctx->big_list.p, *nsb = (uint32_t *)ctx->nsb.p, *npb = (uint32_t *)ctx->npb.p;
-    Row32 *part = (Row32 *)ctx->part.p;
-
-    CU(cudaMemsetAsync(nsb, 0, (size_t)Bl * 4, st));
-    CU(cudaMemsetAsync(npb, 0, (size_t)Bl * 4, st));
-    SegDesc seg{};
-    SeriesEntry *entries = nullptr;
-    uint64_t kept = 0, owned = 0;
-    bool partitioned = false;
-    uint32_t n_ovf = 0;
-    const Row32 *ovf_rows = nullptr;
-    auto offset_cols = [&](uint64_t lo) {
-        ColPtrs ck = c;
-        if (ck.src_ip) ck.src_ip += lo;
-        if (ck.dst_ip) ck.dst_ip += lo;
-        if (ck.src_port) ck.src_port += lo;
-        if (ck.dst_port) ck.dst_port += lo;
-        if (ck.proto) ck.proto += lo;
-        if (ck.flow_start) ck.flow_start += lo;
-        if (ck.flow_end) ck.flow_end += lo;
-        if (ck.value) ck.value += lo;
-        if (ck.src_ns) ck.src_ns += lo;
-        if (ck.dst_ns) ck.dst_ns += lo;
-        return ck;
-    };
     // ---- single GPU, optimistic partition: no histogram pass.  Bucket b owns a fixed slot of kGroupCap rows; a
     // row that finds its slot full goes to the overflow list, and such buckets take the spill path.  With host input
     // the scatter of H2D chunk i runs while chunk i+1 is on the bus.  Falls back to the exact two-pass partition
     // when the overflow list fills up (heavily skewed tables).
-    constexpr uint32_t kSlot = kGroupCap;      // = the largest shared-memory class: overflow is as rare as a spill was
-    const uint64_t slot_rows = (uint64_t)B * kSlot;
-    if (world == 1 && ctx->optimistic && R > 0 && slot_rows * sizeof(Row32) <= (64ull << 30)) {
+    bool local_slots(Partition &p)
+    {
+        constexpr uint32_t kSlot = kGroupCap;      // = the largest shared-memory class: overflow is as rare as a spill was
         const uint64_t ovf_cap = std::max<uint64_t>(1u << 20, R / 32);
-        ensure(ctx->part, slot_rows * sizeof(Row32));
-        ensure(ctx->ovf, ovf_cap * sizeof(Row32));
-        part = (Row32 *)ctx->part.p;
-        Row32 *ovf = (Row32 *)ctx->ovf.p;
+        Row32 *part = (Row32 *)ensure(ctx->part, (uint64_t)B * kSlot * sizeof(Row32));
+        Row32 *ovf = (Row32 *)ensure(ctx->ovf, ovf_cap * sizeof(Row32));
         CU(cudaMemsetAsync(cursor, 0, (size_t)B * 4, st));
         mark(-1);
-        if (host_input) {
-            for (int k = 0; k < nchunks; k++) {
-                uint64_t lo, hi;
-                chunk_range(k, lo, hi);
-                CU(cudaStreamWaitEvent(st, ctx->chunk_ev[k], 0));
-                if (hi <= lo) continue;
-                CU(launch_scatter(st, offset_cols(lo), hi - lo, f, logB, cursor, part, kSlot, ovf, (uint32_t)ovf_cap,
-                                  d_stats + ST_OVF)); launches++;
-            }
-            mark(TAD_PHASE_H2D);          // copy + overlapped scatter of all chunks
-        } else {
-            CU(launch_scatter(st, c, R, f, logB, cursor, part, kSlot, ovf, (uint32_t)ovf_cap, d_stats + ST_OVF)); launches++;
-            mark(TAD_PHASE_SCATTER);
-        }
+        over_input(TAD_PHASE_SCATTER, [&](const ColPtrs &ck, uint64_t n) {
+            return launch_scatter(st, ck, n, f, logB, cursor, part, kSlot, ovf, (uint32_t)ovf_cap, d_stats + ST_OVF);
+        });
         // arrival counts -> (virtual) bucket offsets, capacity-class lists, list of over-full buckets
         CU(launch_bucket_scan(st, cursor, offsets, hist /* unused cursor copy */, B, kSlot, big_list, big_base, cls_list,
                               d_stats, ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
         mark(TAD_PHASE_SCAN);
-        CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        read_stats();
         if (ctx->h_stats[ST_OVF] <= ovf_cap) {
-            partitioned = true;
-            n_ovf = ctx->h_stats[ST_OVF];
-            ovf_rows = ovf;
-            kept = owned = ctx->h_stats[ST_KEPT];
-            seg.nseg = 1;
-            seg.base[0] = part;
-            seg.off[0] = offsets;
-            seg.stride = kSlot;
-            ensure(ctx->entries, (owned ? owned : 1) * sizeof(SeriesEntry));
-            entries = static_cast<SeriesEntry *>(ctx->entries.p);
-        } else {
-            CU(cudaMemsetAsync(d_stats, 0, 64 * sizeof(uint32_t), st));      // discard; redo exactly
+            p.n_ovf = ctx->h_stats[ST_OVF];
+            p.ovf_rows = ovf;
+            p.kept = p.owned = ctx->h_stats[ST_KEPT];
+            p.seg.nseg = 1; p.seg.base[0] = part; p.seg.off[0] = offsets; p.seg.stride = kSlot;
+            p.entries = use_entries(p.owned);
+            return true;
         }
+        CU(cudaMemsetAsync(d_stats, 0, 64 * sizeof(uint32_t), st));      // discard; redo exactly
+        return false;
     }
-
     // ---- exported buffer + peer mappings (multi-GPU peer pull) -----------------------------------------------------------
-    auto gather16 = [&]() {        // blocking 128-byte all-gather through pinned memory (rare: regrow, exact-path row counts)
-        CU(cudaMemcpyAsync(d_small, ctx->h_small, 16 * 8, cudaMemcpyHostToDevice, st));
-        if (nccl_allgather(&ctx->nccl, d_small, d_small + 16, 16 * 8, st)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
-        CU(cudaMemcpyAsync(ctx->h_small + 16, d_small + 16, 16 * 8 * world, cudaMemcpyDeviceToHost, st));
+    void gather16()        // blocking 128-byte all-gather through pinned memory (rare: regrow, exact-path row counts)
+    {
+        CU(cudaMemcpyAsync(d_small + kSlotSend, ctx->h_small + kSlotSend, 16 * 8, cudaMemcpyHostToDevice, st));
+        allgather(d_small + kSlotSend, d_small + kSlotGather16, 16 * 8);
+        CU(cudaMemcpyAsync(ctx->h_small + kSlotGather16, d_small + kSlotGather16, 16 * 8 * world, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
-    };
+    }
     // Every rank calls this with the SAME `need` in the same job (it depends only on values all ranks share), so all ranks
     // regrow together: unmap, barrier (nobody maps a buffer that is about to be freed), reallocate, exchange the IPC
     // handles, map.  First job or a larger table only.
-    auto ensure_exported = [&](size_t need) {
+    void ensure_exported(size_t need)
+    {
         // the decision must be the same on every rank: it is taken on the size the ranks last agreed on, not on the local
         // capacity (which may differ when one rank's allocation fell back to the exact size under memory pressure)
         if (need <= ctx->x_agreed && ctx->peers_mapped) return;
@@ -568,20 +610,20 @@ void run_job(tad_ctx *ctx, tad_job *job)
         for (int r = 0; r < world; r++)
             if (ctx->peer_x[r]) { CU(cudaIpcCloseMemHandle(ctx->peer_x[r])); ctx->peer_x[r] = nullptr; }
         ctx->peers_mapped = false;
-        memset(ctx->h_small, 0, 16 * 8);
+        memset(ctx->h_small + kSlotSend, 0, 16 * 8);
         gather16();
         ensure(ctx->xbuf, need);
         cudaIpcMemHandle_t mine;
         CU(cudaIpcGetMemHandle(&mine, ctx->xbuf.p));
-        memset(ctx->h_small, 0, 16 * 8);
-        ctx->h_small[0] = ctx->xbuf.cap;
-        memcpy(ctx->h_small + 2, &mine, sizeof(mine));
+        memset(ctx->h_small + kSlotSend, 0, 16 * 8);
+        ctx->h_small[kSlotSend] = ctx->xbuf.cap;
+        memcpy(ctx->h_small + kSlotSend + 2, &mine, sizeof(mine));
         gather16();
         for (int r = 0; r < world; r++) {
             if (r == me) continue;
             cudaIpcMemHandle_t h;
-            memcpy(&h, ctx->h_small + 16 + 16 * r + 2, sizeof(h));
-            if (ctx->h_small[16 + 16 * r] < need) fail(TAD_ERR_INTERNAL, "rank %d exports a smaller partition buffer", r);
+            memcpy(&h, ctx->h_small + kSlotGather16 + 16 * r + 2, sizeof(h));
+            if (ctx->h_small[kSlotGather16 + 16 * r] < need) fail(TAD_ERR_INTERNAL, "rank %d exports a smaller partition buffer", r);
             cudaError_t e = cudaIpcOpenMemHandle(&ctx->peer_x[r], h, cudaIpcMemLazyEnablePeerAccess);
             if (e != cudaSuccess) {
                 cudaGetLastError();
@@ -592,43 +634,28 @@ void run_job(tad_ctx *ctx, tad_job *job)
         }
         ctx->peers_mapped = true;
         ctx->x_agreed = need;
-    };
+    }
     // ---- several GPUs, optimistic partition + peer pull ---------------------------------------------------------------
     // Every rank scatters its rows into fixed-capacity slots of ALL global buckets (slot = kGroupCap / world rows: a
     // source holds 1/world of a bucket on average) inside a buffer its peers have mapped with CUDA IPC.  One 8-byte
     // all-gather after the scatter is the barrier "every rank's slots are complete" and carries the overflow counts: if
-    // any slot overflowed anywhere, all ranks take the exact path below (same decision everywhere: it is made on the
+    // any slot overflowed anywhere, all ranks take the exact path (same decision everywhere: it is made on the
     // gathered data).  Otherwise each rank reads the arrival counters of its bucket range out of the peers' buffers and
     // its group kernel pulls the rows themselves, segment by segment, with the bulk copies it issues anyway.
-    const uint32_t slotM = std::max<uint32_t>(256u, (uint32_t)kGroupCap / (uint32_t)world);
-    const size_t x_cnt_bytes = (((size_t)B * 4) + 65535) & ~size_t(65535);
-    const size_t x_need = x_cnt_bytes + (size_t)B * slotM * sizeof(Row32);
-    bool sync_at_end = false;
-    if (world > 1 && ctx->peer_pull && ctx->optimistic && R_total > 0 && (uint64_t)B * slotM <= (1ull << 31) &&
-        x_need <= ctx->x_budget) {
+    bool peer_slots(Partition &p, size_t x_need)
+    {
         ensure_exported(x_need);
         uint32_t *xcursor = static_cast<uint32_t *>(ctx->xbuf.p);
         Row32 *xpart = reinterpret_cast<Row32 *>(static_cast<char *>(ctx->xbuf.p) + x_cnt_bytes);
-        ensure(ctx->xcnt, (size_t)Bl * 4 * world);
-        ensure(ctx->xtotal, (size_t)Bl * 4);
-        uint32_t *xcnt = (uint32_t *)ctx->xcnt.p, *xtotal = (uint32_t *)ctx->xtotal.p;
+        uint32_t *xcnt = (uint32_t *)ensure(ctx->xcnt, (size_t)Bl * 4 * world);
+        uint32_t *xtotal = (uint32_t *)ensure(ctx->xtotal, (size_t)Bl * 4);
         CU(cudaMemsetAsync(xcursor, 0, (size_t)B * 4, st));
         mark(-1);
-        if (host_input) {
-            for (int k = 0; k < nchunks; k++) {
-                uint64_t lo, hi;
-                chunk_range(k, lo, hi);
-                CU(cudaStreamWaitEvent(st, ctx->chunk_ev[k], 0));
-                if (hi <= lo) continue;
-                CU(launch_scatter(st, offset_cols(lo), hi - lo, f, logB, xcursor, xpart, slotM, nullptr, 0, d_stats + ST_OVF)); launches++;
-            }
-            mark(TAD_PHASE_H2D);          // copy + overlapped scatter of all chunks
-        } else {
-            CU(launch_scatter(st, c, R, f, logB, xcursor, xpart, slotM, nullptr, 0, d_stats + ST_OVF)); launches += R ? 1 : 0;
-            mark(TAD_PHASE_SCATTER);
-        }
+        over_input(TAD_PHASE_SCATTER, [&](const ColPtrs &ck, uint64_t n) {
+            return launch_scatter(st, ck, n, f, logB, xcursor, xpart, slotM, nullptr, 0, d_stats + ST_OVF);
+        });
         // barrier + overflow agreement: {overflow rows, -} of every rank
-        if (nccl_allgather(&ctx->nccl, d_stats + ST_OVF, d_small + 32, 8, st)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
+        allgather(d_stats + ST_OVF, d_small + kSlotOvf, 8);
         mark(TAD_PHASE_SYNC);
         PeerCounters pc{};
         for (int r = 0; r < world; r++) pc.p[r] = r == me ? xcursor : static_cast<const uint32_t *>(ctx->peer_x[r]);
@@ -637,104 +664,78 @@ void run_job(tad_ctx *ctx, tad_job *job)
         CU(launch_bucket_scan(st, xtotal, offsets, cursor, Bl, kGroupCap, big_list, big_base, cls_list, d_stats,
                               ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
         mark(TAD_PHASE_SCAN);
-        CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(ctx->h_small + 32, d_small + 32, 8 * world, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        CU(cudaMemcpyAsync(ctx->h_small + kSlotOvf, d_small + kSlotOvf, 8 * world, cudaMemcpyDeviceToHost, st));
+        read_stats();
         check_cancel();
         uint64_t any_ovf = 0;
-        for (int r = 0; r < world; r++) any_ovf += (uint32_t)ctx->h_small[32 + r];
-        sync_at_end = true;       // peers may still read this rank's slots: no rank starts its next job before all are done
+        for (int r = 0; r < world; r++) any_ovf += (uint32_t)ctx->h_small[kSlotOvf + r];
         if (any_ovf == 0) {
-            partitioned = true;
-            kept = ctx->h_stats[ST_LOCALKEPT];
-            owned = ctx->h_stats[ST_KEPT];
-            seg.nseg = world;
-            seg.stride = slotM;
-            seg.b_lo = b_lo;
-            for (int r = 0; r < world; r++) {
-                const char *xb = r == me ? static_cast<const char *>(ctx->xbuf.p) : static_cast<const char *>(ctx->peer_x[r]);
-                seg.base[r] = reinterpret_cast<const Row32 *>(xb + x_cnt_bytes);
-                seg.off[r] = xcnt + (size_t)r * Bl;
-            }
-            ensure(ctx->entries, (owned ? owned : 1) * sizeof(SeriesEntry));
-            entries = static_cast<SeriesEntry *>(ctx->entries.p);
-        } else {
-            CU(cudaMemsetAsync(d_stats, 0, 64 * sizeof(uint32_t), st));      // discard; redo exactly (every rank does)
+            p.sync_at_end = true;       // peers may still read this rank's slots: no rank starts its next job before all are done
+            p.kept = ctx->h_stats[ST_LOCALKEPT];
+            p.owned = ctx->h_stats[ST_KEPT];
+            p.seg.nseg = world; p.seg.stride = slotM; p.seg.b_lo = b_lo;
+            for (int r = 0; r < world; r++) { p.seg.base[r] = peer_rows(r); p.seg.off[r] = xcnt + (size_t)r * Bl; }
+            p.entries = use_entries(p.owned);
+            return true;
         }
+        CU(cudaMemsetAsync(d_stats, 0, 64 * sizeof(uint32_t), st));      // discard; redo exactly (every rank does)
+        return false;
     }
-    if (world == 1 && !partitioned) {
+    // ---- single GPU, exact partition: histogram, scan, scatter; also the fallback of the optimistic one -----------------
+    Partition exact_local()
+    {
+        Row32 *part = (Row32 *)ctx->part.p;
         CU(cudaMemsetAsync(hist, 0, (size_t)B * 4, st));
         mark(-1);
-        if (host_input) {
-            for (int k = 0; k < nchunks; k++) {
-                uint64_t lo, hi;
-                chunk_range(k, lo, hi);
-                CU(cudaStreamWaitEvent(st, ctx->chunk_ev[k], 0));
-                if (hi <= lo) continue;
-                CU(launch_hist(st, offset_cols(lo), hi - lo, f, logB, hist)); launches++;
-            }
-            mark(TAD_PHASE_H2D);          // copy + overlapped histogram of all chunks
-        } else {
-            CU(launch_hist(st, c, R, f, logB, hist)); launches += R ? 1 : 0;
-            mark(TAD_PHASE_HIST);
-        }
-        // single GPU: these are the final bucket offsets; multi GPU: offsets inside the local send buffer
-        CU(launch_bucket_scan(st, hist, offsets, cursor, B, world > 1 ? 0xffffffffu : (uint32_t)kGroupCap, big_list, big_base,
-                              world > 1 ? nullptr : cls_list, d_stats, ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
+        over_input(TAD_PHASE_HIST, [&](const ColPtrs &ck, uint64_t n) { return launch_hist(st, ck, n, f, logB, hist); });
+        CU(launch_bucket_scan(st, hist, offsets, cursor, B, (uint32_t)kGroupCap, big_list, big_base, cls_list, d_stats,
+                              ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
         mark(TAD_PHASE_SCAN);
         CU(launch_scatter(st, c, R, f, logB, cursor, part)); launches += R ? 1 : 0;
         mark(TAD_PHASE_SCATTER);
-        CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        kept = owned = ctx->h_stats[ST_KEPT];
-        seg.nseg = 1;
-        seg.base[0] = part;
-        seg.off[0] = offsets;
-        entries = reinterpret_cast<SeriesEntry *>(part);      // in place over the staged bucket rows
-    } else if (world > 1 && !partitioned) {
-        // ---- multi GPU, exact partition: K row chunks; chunk c is sent over NVLink (comm stream) while chunk c+1 is scattered ------
-        // chunked (overlapped) exchange pays off at N = 2 (measured 11.5 -> 9.6 ms); at N >= 4 the NVLink all-to-all is
-        // longer than the scatter it could hide behind and the extra segments cost the group kernel more than is won
-        // With peer pull (default) the exact partition is written into the EXPORTED buffer and the owners' group kernels read
-        // their segments straight out of the peers' copies: no receive buffer, no all-to-all (and no chunking: K = 1).
+        read_stats();
+        Partition p;
+        p.kept = p.owned = ctx->h_stats[ST_KEPT];
+        p.seg.nseg = 1; p.seg.base[0] = part; p.seg.off[0] = offsets;
+        p.entries = reinterpret_cast<SeriesEntry *>(part);      // in place over the staged bucket rows
+        return p;
+    }
+    // ---- multi GPU, exact partition: K row chunks; chunk c is sent over NVLink (comm stream) while chunk c+1 is scattered ------
+    // chunked (overlapped) exchange pays off at N = 2 (measured 11.5 -> 9.6 ms); at N >= 4 the NVLink all-to-all is
+    // longer than the scatter it could hide behind and the extra segments cost the group kernel more than is won
+    // With peer pull (default) the exact partition is written into the EXPORTED buffer and the owners' group kernels read
+    // their segments straight out of the peers' copies: no receive buffer, no all-to-all (and no chunking: K = 1).
+    Partition exact_multi()
+    {
         const bool pull = ctx->peer_pull != 0;
         const int K = pull ? 1 : (R >= ctx->exchange_min_rows && (world == 2 || ctx->exchange_chunks_forced)) ? ctx->exchange_chunks : 1;
-        auto xlo = [&](int cidx) -> uint64_t {
-            if (cidx <= 0) return 0;
-            if (cidx >= K) return R;
-            const uint64_t v = ((R * (uint64_t)cidx / K) + 15) & ~uint64_t(15);
-            return v < R ? v : R;
-        };
         const int NS = world * K;                              // segments: (source rank, chunk)
+        Row32 *part;
         if (pull) {
             // the exported buffer must hold the largest shard: the ranks agree on it (blocking 128-byte all-gather; this path
             // is the fallback for skewed or very large tables, where a host sync more does not matter)
-            memset(ctx->h_small, 0, 16 * 8);
-            ctx->h_small[0] = R;
+            memset(ctx->h_small + kSlotSend, 0, 16 * 8);
+            ctx->h_small[kSlotSend] = R;
             gather16();
             uint64_t max_rows = 1;
-            for (int r = 0; r < world; r++) max_rows = std::max<uint64_t>(max_rows, ctx->h_small[16 + 16 * r]);
+            for (int r = 0; r < world; r++) max_rows = std::max<uint64_t>(max_rows, ctx->h_small[kSlotGather16 + 16 * r]);
             ensure_exported(x_cnt_bytes + max_rows * sizeof(Row32));
             part = reinterpret_cast<Row32 *>(static_cast<char *>(ctx->xbuf.p) + x_cnt_bytes);
         } else {
-            ensure(ctx->part, (R ? R : 1) * sizeof(Row32));
-            part = (Row32 *)ctx->part.p;
+            part = (Row32 *)ensure(ctx->part, (R ? R : 1) * sizeof(Row32));
         }
-        ensure(ctx->hist, (size_t)B * 4 * K);
-        ensure(ctx->offsets, ((size_t)B + 1) * 4 * K);
-        ensure(ctx->cursor, (size_t)B * 4 * K);
-        ensure(ctx->hist_all, (size_t)B * 4 * NS);
-        ensure(ctx->seg_off, ((size_t)Bl + 1) * 4 * NS);
-        ensure(ctx->seg_total, (size_t)Bl * 4);
-        hist = (uint32_t *)ctx->hist.p; offsets = (uint32_t *)ctx->offsets.p; cursor = (uint32_t *)ctx->cursor.p;
-        uint32_t *hist_all = (uint32_t *)ctx->hist_all.p, *seg_off = (uint32_t *)ctx->seg_off.p;
-        uint32_t *seg_total = (uint32_t *)ctx->seg_total.p;
+        hist = (uint32_t *)ensure(ctx->hist, (size_t)B * 4 * K);
+        offsets = (uint32_t *)ensure(ctx->offsets, ((size_t)B + 1) * 4 * K);
+        cursor = (uint32_t *)ensure(ctx->cursor, (size_t)B * 4 * K);
+        uint32_t *hist_all = (uint32_t *)ensure(ctx->hist_all, (size_t)B * 4 * NS);
+        uint32_t *seg_off = (uint32_t *)ensure(ctx->seg_off, ((size_t)Bl + 1) * 4 * NS);
+        uint32_t *seg_total = (uint32_t *)ensure(ctx->seg_total, (size_t)Bl * 4);
         CU(cudaMemsetAsync(hist, 0, (size_t)B * 4 * K, st));
         if (host_input)
             for (int k = 0; k < nchunks; k++) CU(cudaStreamWaitEvent(st, ctx->chunk_ev[k], 0));
         mark(TAD_PHASE_H2D);
         for (int cx = 0; cx < K; cx++) {
-            const uint64_t lo = xlo(cx), hi = xlo(cx + 1);
+            const uint64_t lo = split(cx, K), hi = split(cx + 1, K);
             if (hi > lo) { CU(launch_hist(st, offset_cols(lo), hi - lo, f, logB, hist + (size_t)cx * B)); launches++; }
         }
         mark(TAD_PHASE_HIST);
@@ -744,183 +745,164 @@ void run_job(tad_ctx *ctx, tad_job *job)
         }
         mark(TAD_PHASE_SCAN);
         // every rank learns every (rank, chunk) histogram: segment offsets of the owned bucket range, receive sizes
-        if (nccl_allgather(&ctx->nccl, hist, hist_all, (size_t)B * 4 * K, st)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
-        CU(launch_segment_scan(st, hist_all, B, b_lo, Bl, NS, seg_off, seg_total, d_small, pull ? d_small + 40 : nullptr)); launches += 2;
-        CU(cudaMemcpyAsync(ctx->h_small, d_small, 8 * NS, cudaMemcpyDeviceToHost, st));
-        if (pull) CU(cudaMemcpyAsync(ctx->h_small + 40, d_small + 40, 8 * NS, cudaMemcpyDeviceToHost, st));
+        allgather(hist, hist_all, (size_t)B * 4 * K);
+        CU(launch_segment_scan(st, hist_all, B, b_lo, Bl, NS, seg_off, seg_total, d_small + kSlotSegRows,
+                               pull ? d_small + kSlotFront : nullptr)); launches += 2;
+        CU(cudaMemcpyAsync(ctx->h_small + kSlotSegRows, d_small + kSlotSegRows, 8 * NS, cudaMemcpyDeviceToHost, st));
+        if (pull) CU(cudaMemcpyAsync(ctx->h_small + kSlotFront, d_small + kSlotFront, 8 * NS, cudaMemcpyDeviceToHost, st));
         for (int cx = 0; cx < K; cx++)        // send boundaries of chunk cx: offsets_cx[p * Bl], p = 0..world
-            CU(cudaMemcpy2DAsync(ctx->h_small + 64 + cx * (kMaxRanks + 1), 8, offsets + (size_t)cx * (B + 1), (size_t)Bl * 4, 4,
+            CU(cudaMemcpy2DAsync(ctx->h_small + kSlotSendLo + cx * (kMaxRanks + 1), 8, offsets + (size_t)cx * (B + 1), (size_t)Bl * 4, 4,
                                  world + 1, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         check_cancel();
-        uint64_t recv_off[kMaxSeg], recv_total = 0, send_lo[kMaxXChunks][kMaxRanks + 1];
+        const unsigned long long *seg_rows = ctx->h_small + kSlotSegRows;
+        SegDesc seg{};
+        uint64_t kept = 0, owned = 0;
+        bool sync_at_end = false;
+        uint64_t recv_off[kMaxSeg], recv_total = 0, send_lo[kMaxXChunks][kMaxRanks + 1] = {};
         for (int sgi = 0; sgi < NS; sgi++) {
             recv_off[sgi] = recv_total;
-            if (sgi / K != me) recv_total += ctx->h_small[sgi] * 32;
-            owned += ctx->h_small[sgi];
+            if (sgi / K != me) recv_total += seg_rows[sgi] * 32;
+            owned += seg_rows[sgi];
         }
         for (int cx = 0; cx < K; cx++) {
-            for (int p = 0; p <= world; p++) send_lo[cx][p] = (uint32_t)ctx->h_small[64 + cx * (kMaxRanks + 1) + p];
+            for (int p = 0; p <= world; p++) send_lo[cx][p] = (uint32_t)ctx->h_small[kSlotSendLo + cx * (kMaxRanks + 1) + p];
             kept += send_lo[cx][world];
         }
         if (owned >= (1ull << 32) - 1) fail(TAD_ERR_INVALID_ARG, "more than 2^32-2 rows owned by one GPU after the exchange");
-        cudaStream_t cs = ctx->copy_stream;
         if (pull) {
+            // peer pull: the owners' group kernels read their segments out of the exported partitions
             CU(launch_scatter(st, c, R, f, logB, cursor, part)); launches += R ? 1 : 0;
             mark(TAD_PHASE_SCATTER);
-            // barrier: every rank's exact partition is complete
-            if (nccl_allgather(&ctx->nccl, d_small + 48, d_small + 56, 8, st)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
+            nccl_ok(barrier(ctx));              // every rank's exact partition is complete
             mark(TAD_PHASE_SYNC);
             seg.nseg = world;
             for (int r = 0; r < world; r++) {
-                const char *xb = r == me ? static_cast<const char *>(ctx->xbuf.p) : static_cast<const char *>(ctx->peer_x[r]);
-                seg.base[r] = reinterpret_cast<const Row32 *>(xb + x_cnt_bytes) + ctx->h_small[40 + r];   // rows in front of my range
+                seg.base[r] = peer_rows(r) + ctx->h_small[kSlotFront + r];   // rows in front of my range
                 seg.off[r] = seg_off + (size_t)r * (Bl + 1);
             }
             sync_at_end = true;
         } else {
-        ensure(ctx->exch, recv_total ? recv_total : 32);
-        for (int cx = 0; cx < K; cx++) {
-            const uint64_t lo = xlo(cx), hi = xlo(cx + 1);
-            if (hi > lo) { CU(launch_scatter(st, offset_cols(lo), hi - lo, f, logB, cursor + (size_t)cx * B, part + lo)); launches++; }
-            CU(cudaEventRecord(ctx->x_ev[cx], st));
-            CU(cudaStreamWaitEvent(cs, ctx->x_ev[cx], 0));
-            uint64_t so[kMaxRanks], sb[kMaxRanks], ro[kMaxRanks], rb[kMaxRanks];
-            for (int p = 0; p < world; p++) {
-                so[p] = (lo + send_lo[cx][p]) * 32;
-                sb[p] = (send_lo[cx][p + 1] - send_lo[cx][p]) * 32;
-                ro[p] = recv_off[p * K + cx];
-                rb[p] = ctx->h_small[p * K + cx] * 32;
+            // NCCL all-to-all (TAD_PEER_PULL=0): chunk cx is sent on the copy stream while chunk cx+1 is scattered
+            cudaStream_t cs = ctx->copy_stream;
+            ensure(ctx->exch, recv_total ? recv_total : 32);
+            for (int cx = 0; cx < K; cx++) {
+                const uint64_t lo = split(cx, K), hi = split(cx + 1, K);
+                if (hi > lo) { CU(launch_scatter(st, offset_cols(lo), hi - lo, f, logB, cursor + (size_t)cx * B, part + lo)); launches++; }
+                CU(cudaEventRecord(ctx->x_ev[cx], st));
+                CU(cudaStreamWaitEvent(cs, ctx->x_ev[cx], 0));
+                uint64_t so[kMaxRanks], sb[kMaxRanks], ro[kMaxRanks], rb[kMaxRanks];
+                for (int p = 0; p < world; p++) {
+                    so[p] = (lo + send_lo[cx][p]) * 32;
+                    sb[p] = (send_lo[cx][p + 1] - send_lo[cx][p]) * 32;
+                    ro[p] = recv_off[p * K + cx];
+                    rb[p] = seg_rows[p * K + cx] * 32;
+                }
+                nccl_ok(nccl_alltoallv(&ctx->nccl, part, so, sb, ctx->exch.p, ro, rb, cs));
             }
-            if (nccl_alltoallv(&ctx->nccl, part, so, sb, ctx->exch.p, ro, rb, cs)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
-        }
-        mark(TAD_PHASE_SCATTER);
-        CU(cudaEventRecord(ctx->x_ev[K], cs));
-        CU(cudaStreamWaitEvent(st, ctx->x_ev[K], 0));
-        seg.nseg = NS;
-        for (int sgi = 0; sgi < NS; sgi++) {
-            const int r = sgi / K, cx = sgi % K;
-            seg.base[sgi] = r == me ? part + xlo(cx) + send_lo[cx][me]
-                                    : reinterpret_cast<const Row32 *>((const char *)ctx->exch.p + recv_off[sgi]);
-            seg.off[sgi] = seg_off + (size_t)sgi * (Bl + 1);
-        }
+            mark(TAD_PHASE_SCATTER);
+            CU(cudaEventRecord(ctx->x_ev[K], cs));
+            CU(cudaStreamWaitEvent(st, ctx->x_ev[K], 0));
+            seg.nseg = NS;
+            for (int sgi = 0; sgi < NS; sgi++) {
+                const int r = sgi / K, cx = sgi % K;
+                seg.base[sgi] = r == me ? part + split(cx, K) + send_lo[cx][me]
+                                        : reinterpret_cast<const Row32 *>((const char *)ctx->exch.p + recv_off[sgi]);
+                seg.off[sgi] = seg_off + (size_t)sgi * (Bl + 1);
+            }
         }
         // final (virtual) bucket offsets of the owned range, oversized-bucket list, capacity-class lists
         CU(launch_bucket_scan(st, seg_total, offsets, cursor, Bl, kGroupCap, big_list, big_base, cls_list, d_stats,
                               ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
         mark(TAD_PHASE_EXCHANGE);           // = the part of the exchange NOT hidden behind the scatter
-        CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        ensure(ctx->entries, (owned ? owned : 1) * sizeof(SeriesEntry));
-        entries = static_cast<SeriesEntry *>(ctx->entries.p);
+        read_stats();
+        return Partition{seg, use_entries(owned), kept, owned, nullptr, 0, sync_at_end};
     }
-    check_cancel();
-    const uint32_t n_big = ctx->h_stats[ST_NBIG];
-    const uint64_t big_rows = ctx->h_stats[ST_BIGROWS];
-    set_progress(job, TAD_STATE_RUNNING, 3);    // ingest, partition, exchange
-
-    // ---- group ------------------------------------------------------------------------------
-    const uint64_t cap_rows = owned ? owned : 1;
-    ensure(ctx->csr_v, cap_rows * 8 + 64);       // + one sector: the direct detector reads whole 32-byte sectors
-    ensure(ctx->csr_t, cap_rows * 4);
-    uint64_t *csr_v = (uint64_t *)ctx->csr_v.p;
-    uint32_t *csr_t = (uint32_t *)ctx->csr_t.p;
-    uint32_t *csr_p = nullptr;
-    if (sp.algo == TAD_ALGO_DBSCAN) {
-        ensure(ctx->csr_p, cap_rows * 4);
-        csr_p = (uint32_t *)ctx->csr_p.p;
-    }
-    mark(-1);
+    // ---- group (+ spill) ------------------------------------------------------------------
+    void group(const Partition &p, uint32_t n_big, uint64_t big_rows)
     {
+        const uint64_t cap_rows = p.owned ? p.owned : 1;
+        csr_v = (uint64_t *)ensure(ctx->csr_v, cap_rows * 8 + 64);       // + one sector: the direct detector reads whole 32-byte sectors
+        csr_t = (uint32_t *)ensure(ctx->csr_t, cap_rows * 4);
+        if (sp.algo == TAD_ALGO_DBSCAN) csr_p = (uint32_t *)ensure(ctx->csr_p, cap_rows * 4);
+        mark(-1);
         int l = 0;
         const uint32_t n_cls[3] = {ctx->h_stats[ST_NCLS0], ctx->h_stats[ST_NCLS1], ctx->h_stats[ST_NCLS2]};
         if (ctx->sort_classes) {
             // class lists in ascending bucket order: concurrently running CTAs then touch neighbouring slots / csr stretches
-            const size_t need = sort_lists_scratch_bytes(Bl);
-            ensure(ctx->sortb, need);
+            ensure(ctx->sortb, sort_lists_scratch_bytes(Bl));
             int bits = 1;
             while ((1u << bits) < Bl && bits < 32) bits++;
             for (int k = 0; k < 3; k++)
                 if (n_cls[k] > 1) { CU(sort_bucket_list(st, cls_list + (size_t)k * Bl, n_cls[k], bits, ctx->sortb.p, ctx->sortb.cap)); launches += 3; }
         }
-        CU(launch_group(st, seg, entries, offsets, Bl, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb, sp.reducer, &l));
+        CU(launch_group(st, p.seg, p.entries, offsets, Bl, cls_list, n_cls, csr_v, csr_t, csr_p, nsb, npb, sp.reducer, &l));
         launches += l;
-    }
-    mark(TAD_PHASE_GROUP);
-    if (n_big) {
-        const size_t need = spill_scratch_bytes(big_rows);
-        ensure(ctx->spill, need);
-        int l = 0;
-        CU(run_spill(st, seg, entries, offsets, big_list, big_base, n_big, big_rows, ctx->spill.p, ctx->spill.cap, csr_v, csr_t,
-                     nsb, npb, sp.reducer, &l, ovf_rows, n_ovf));
-        launches += l;
-        mark(TAD_PHASE_SPILL);
-    }
-    ensure(ctx->sbase, sbase_words(Bl, cap_rows) * 4);      // series base per bucket + bucket hint per 32 series
-    uint32_t *sbase = (uint32_t *)ctx->sbase.p;
-    CU(launch_series_scan(st, nsb, npb, sbase, Bl, d_stats, ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
-    CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    check_cancel();
-    const uint32_t S = ctx->h_stats[ST_SERIES];
-    const uint64_t points = ctx->h_stats[ST_POINTS];
-    set_progress(job, TAD_STATE_RUNNING, 4);
-
-    // ---- detect -----------------------------------------------------------------------------
-    const bool emit_all = (sp.flags & TAD_FLAG_EMIT_ALL) != 0;
-    uint64_t out_cap = emit_all ? points : (points / 8 + (1u << 16));
-    if (out_cap > points) out_cap = points;
-    if (out_cap == 0) out_cap = 1;
-    uint64_t out_rows = 0;
-    OutLayout L{};
-    OutCols oc{};
-    for (int attempt = 0; attempt < 3; attempt++) {
-        L = out_layout(out_cap);
-        ensure(ctx->outb, L.total);
-        oc = out_cols(ctx->outb.p, L);
-        CU(cudaMemsetAsync(d_stats + ST_OUTCOUNT, 0, 4, st));
-        mark(-1);
-        if (sp.algo == TAD_ALGO_EWMA) {
-            CU(launch_detect_ewma(st, entries, offsets, sbase, Bl, S, csr_v, csr_t, oc, (uint32_t)out_cap, d_stats, emit_all));
-            launches += S ? 1 : 0;
-        } else if (sp.algo == TAD_ALGO_DBSCAN) {
-            ensure(ctx->dbx, cap_rows * 4);         // prefix count of core points, per point slot
-            ensure(ctx->dbi, cap_rows);             // noise flag, per point slot
-            CU(launch_detect_dbscan(st, entries, offsets, sbase, Bl, S, csr_v, csr_t, csr_p, (uint32_t *)ctx->dbx.p,
-                                    (uint8_t *)ctx->dbi.p, oc, (uint32_t)out_cap, d_stats, emit_all));
-            launches += S ? 1 : 0;
-        } else if (sp.algo == TAD_ALGO_ARIMA) {
-            ensure(ctx->ar_y, cap_rows * 8);
-            ensure(ctx->ar_pred, cap_rows * 8);
-            ensure(ctx->ar_lam, ((size_t)S + 1) * 8);
-            CU(launch_detect_arima(st, entries, offsets, sbase, Bl, S, csr_v, csr_t, (double *)ctx->ar_y.p,
-                                   (double *)ctx->ar_pred.p, (double *)ctx->ar_lam.p, attempt == 0, oc, (uint32_t)out_cap,
-                                   d_stats, emit_all));
-            launches += S ? (attempt == 0 ? 3 : 1) : 0;
-        } else {
-            fail(TAD_ERR_UNSUPPORTED, "algorithm %d is not implemented by this build", sp.algo);
+        mark(TAD_PHASE_GROUP);
+        if (n_big) {
+            ensure(ctx->spill, spill_scratch_bytes(big_rows));
+            l = 0;
+            CU(run_spill(st, p.seg, p.entries, offsets, big_list, big_base, n_big, big_rows, ctx->spill.p, ctx->spill.cap, csr_v,
+                         csr_t, nsb, npb, sp.reducer, &l, p.ovf_rows, p.n_ovf));
+            launches += l;
+            mark(TAD_PHASE_SPILL);
         }
-        mark(TAD_PHASE_DETECT);
-        CU(cudaMemcpyAsync(ctx->h_stats, d_stats, ST_COUNT * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        out_rows = ctx->h_stats[ST_OUTCOUNT];
-        if (out_rows <= out_cap) break;
-        out_cap = out_rows;                 // capacity guess too small: rerun detect (idempotent)
-        if (attempt == 2) fail(TAD_ERR_INTERNAL, "result capacity did not converge");
     }
-    check_cancel();
-    set_progress(job, TAD_STATE_RUNNING, 5);
-    if (sync_at_end) {
-        // end-of-job barrier of the peer-pull path: my slots and counters may be overwritten (next job) only after every
-        // peer's group kernel has read them; its wait is the ranks' arrival skew, accounted as TAD_PHASE_SYNC
-        mark(-1);
-        if (nccl_allgather(&ctx->nccl, d_small + 48, d_small + 56, 8, st)) fail(TAD_ERR_NCCL, "%s", nccl_last_error());
-        mark(TAD_PHASE_SYNC);
-    }
-
-    // ---- egress: result rows -> pinned host memory -------------------------------------------
-    mark(-1);
+    // ---- series scan: series base per bucket; series and point counts -> h_stats ------------
+    void series_scan(uint64_t owned)
     {
+        sbase = (uint32_t *)ensure(ctx->sbase, sbase_words(Bl, owned ? owned : 1) * 4);   // + bucket hint per 32 series
+        CU(launch_series_scan(st, nsb, npb, sbase, Bl, d_stats, ctx->scan_sync.p, ++ctx->scan_epoch)); launches++;
+        read_stats();
+    }
+    // ---- detect: result rows into the device buffer of layout L; returns their count --------
+    uint64_t detect(const Partition &p, uint32_t S, uint64_t points, OutLayout &L)
+    {
+        const uint64_t cap_rows = p.owned ? p.owned : 1;
+        const bool emit_all = (sp.flags & TAD_FLAG_EMIT_ALL) != 0;
+        uint64_t out_cap = emit_all ? points : (points / 8 + (1u << 16));
+        if (out_cap > points) out_cap = points;
+        if (out_cap == 0) out_cap = 1;
+        uint64_t out_rows = 0;
+        for (int attempt = 0; attempt < 3; attempt++) {
+            L = out_layout(out_cap);
+            ensure(ctx->outb, L.total);
+            const OutCols oc = out_cols(ctx->outb.p, L);
+            CU(cudaMemsetAsync(d_stats + ST_OUTCOUNT, 0, 4, st));
+            mark(-1);
+            if (sp.algo == TAD_ALGO_EWMA) {
+                CU(launch_detect_ewma(st, p.entries, offsets, sbase, Bl, S, csr_v, csr_t, oc, (uint32_t)out_cap, d_stats, emit_all));
+                launches += S ? 1 : 0;
+            } else if (sp.algo == TAD_ALGO_DBSCAN) {
+                ensure(ctx->dbx, cap_rows * 4);         // prefix count of core points, per point slot
+                ensure(ctx->dbi, cap_rows);             // noise flag, per point slot
+                CU(launch_detect_dbscan(st, p.entries, offsets, sbase, Bl, S, csr_v, csr_t, csr_p, (uint32_t *)ctx->dbx.p,
+                                        (uint8_t *)ctx->dbi.p, oc, (uint32_t)out_cap, d_stats, emit_all));
+                launches += S ? 1 : 0;
+            } else if (sp.algo == TAD_ALGO_ARIMA) {
+                ensure(ctx->ar_y, cap_rows * 8);
+                ensure(ctx->ar_pred, cap_rows * 8);
+                ensure(ctx->ar_lam, ((size_t)S + 1) * 8);
+                CU(launch_detect_arima(st, p.entries, offsets, sbase, Bl, S, csr_v, csr_t, (double *)ctx->ar_y.p,
+                                       (double *)ctx->ar_pred.p, (double *)ctx->ar_lam.p, attempt == 0, oc, (uint32_t)out_cap,
+                                       d_stats, emit_all));
+                launches += S ? (attempt == 0 ? 3 : 1) : 0;
+            } else {
+                fail(TAD_ERR_UNSUPPORTED, "algorithm %d is not implemented by this build", sp.algo);
+            }
+            mark(TAD_PHASE_DETECT);
+            read_stats();
+            out_rows = ctx->h_stats[ST_OUTCOUNT];
+            if (out_rows <= out_cap) break;
+            out_cap = out_rows;                 // capacity guess too small: rerun detect (idempotent)
+            if (attempt == 2) fail(TAD_ERR_INTERNAL, "result capacity did not converge");
+        }
+        return out_rows;
+    }
+    // ---- egress: result rows -> pinned host memory -------------------------------------------
+    void egress(const OutLayout &L, uint64_t out_rows)
+    {
+        mark(-1);
         static const size_t w[11] = {8, 8, 8, 4, 4, 4, 4, 2, 2, 1, 1};
         OutLayout HL = out_layout(out_rows ? out_rows : 1);
         job->result_block = take_pinned(ctx, HL.total);
@@ -935,45 +917,69 @@ void run_job(tad_ctx *ctx, tad_job *job)
         job->rows.proto = ho.proto; job->rows.flow_start = ho.flow_start; job->rows.flow_end = ho.flow_end;
         job->rows.stddev = ho.stddev; job->rows.algo_calc = ho.algo_calc; job->rows.throughput = ho.throughput;
         job->rows.anomaly = ho.anomaly;
+        mark(TAD_PHASE_D2H);
+        CU(cudaStreamSynchronize(st));
     }
-    mark(TAD_PHASE_D2H);
-    CU(cudaStreamSynchronize(st));
-
-    // ---- status ---------------------------------------------------------------------------------
-    double phase_ms[TAD_NPHASES] = {0};
-    float total = 0;
-    for (int i = 1; i < nev; i++) {
-        if (ev_phase[i] < 0) continue;
-        float ms = 0;
-        CU(cudaEventElapsedTime(&ms, ctx->ev[i - 1], ctx->ev[i]));
-        phase_ms[ev_phase[i]] += ms;
-    }
-    // device span excludes the H2D/D2H copies: first partition event .. last detect event
-    int first_k = -1, last_k = -1;
-    for (int i = 0; i < nev; i++) {
-        if ((ev_phase[i] == TAD_PHASE_HIST || ev_phase[i] == TAD_PHASE_H2D || ev_phase[i] == TAD_PHASE_SCATTER) && first_k < 0)
-            first_k = i - 1;
-        if (ev_phase[i] == TAD_PHASE_DETECT || (ev_phase[i] == TAD_PHASE_SYNC && last_k >= 0)) last_k = i;
-    }
-    if (first_k >= 0 && last_k > first_k) CU(cudaEventElapsedTime(&total, ctx->ev[first_k], ctx->ev[last_k]));
+    // ---- status: counts, phase times; the job is COMPLETED ---------------------------------------
+    void report(const Partition &p, uint32_t S, uint64_t points, uint64_t out_rows, uint64_t big_rows)
     {
+        double phase_ms[TAD_NPHASES] = {0};
+        float total = 0;
+        for (int i = 1; i < nev; i++) {
+            if (ev_phase[i] < 0) continue;
+            float ms = 0;
+            CU(cudaEventElapsedTime(&ms, ctx->ev[i - 1], ctx->ev[i]));
+            phase_ms[ev_phase[i]] += ms;
+        }
+        // device span excludes the H2D/D2H copies: first partition event .. last detect event
+        int first_k = -1, last_k = -1;
+        for (int i = 0; i < nev; i++) {
+            if ((ev_phase[i] == TAD_PHASE_HIST || ev_phase[i] == TAD_PHASE_H2D || ev_phase[i] == TAD_PHASE_SCATTER) && first_k < 0)
+                first_k = i - 1;
+            if (ev_phase[i] == TAD_PHASE_DETECT || (ev_phase[i] == TAD_PHASE_SYNC && last_k >= 0)) last_k = i;
+        }
+        if (first_k >= 0 && last_k > first_k) CU(cudaEventElapsedTime(&total, ctx->ev[first_k], ctx->ev[last_k]));
         std::lock_guard<std::mutex> lk(job->mu);
         tad_status &s = job->st;
-        s.rows_in = R;
-        s.rows_kept = kept;
-        s.rows_owned = owned;
-        s.points = points;
-        s.series = S;
-        s.result_rows = out_rows;
-        s.spill_rows = big_rows;
-        s.gpu_launches = launches;
-        s.device_ms = total;
+        s.rows_in = R; s.rows_kept = p.kept; s.rows_owned = p.owned;
+        s.points = points; s.series = S; s.result_rows = out_rows; s.spill_rows = big_rows;
+        s.gpu_launches = launches; s.device_ms = total;
         for (int i = 0; i < TAD_NPHASES; i++) s.phase_ms[i] = phase_ms[i];
         s.total_ms = now_ms() - job->t_submit;
-        s.completed_stages = kTotalStages;
-        s.state = TAD_STATE_COMPLETED;
+        s.completed_stages = kTotalStages; s.state = TAD_STATE_COMPLETED;
         job->cv.notify_all();     // last touch of `job` by the worker (tad_release may free it now)
     }
+};
+
+void run_job(tad_ctx *ctx, tad_job *job)
+{
+    JobRun run(ctx, job);
+    run.ingest();
+    run.pick_buckets();
+    const Partition p = run.partition();
+    run.check_cancel();
+    const uint32_t n_big = ctx->h_stats[ST_NBIG];
+    const uint64_t big_rows = ctx->h_stats[ST_BIGROWS];
+    set_progress(job, TAD_STATE_RUNNING, 3);    // ingest, partition, exchange
+    run.group(p, n_big, big_rows);
+    run.series_scan(p.owned);
+    run.check_cancel();
+    const uint32_t S = ctx->h_stats[ST_SERIES];
+    const uint64_t points = ctx->h_stats[ST_POINTS];
+    set_progress(job, TAD_STATE_RUNNING, 4);
+    OutLayout L{};
+    const uint64_t out_rows = run.detect(p, S, points, L);
+    run.check_cancel();
+    set_progress(job, TAD_STATE_RUNNING, 5);
+    if (p.sync_at_end) {
+        // end-of-job barrier of the peer-pull paths: my slots and counters may be overwritten (next job) only after every
+        // peer's group kernel has read them; its wait is the ranks' arrival skew, accounted as TAD_PHASE_SYNC
+        run.mark(-1);
+        nccl_ok(barrier(ctx));
+        run.mark(TAD_PHASE_SYNC);
+    }
+    run.egress(L, out_rows);
+    run.report(p, S, points, out_rows, big_rows);
 }
 
 void worker_main(tad_ctx *ctx)
@@ -1088,7 +1094,6 @@ int tad_init(const tad_config *cfg, tad_ctx **out)
     ctx->cfg.nccl_unique_id = nullptr;
     if (const char *e = getenv("TAD_DEBUG_LOGB")) ctx->debug_logb = atoi(e);
     if (const char *e = getenv("TAD_GROUP_TARGET")) ctx->debug_target = atoi(e);
-    cudaDeviceGetAttribute(&ctx->num_sms, cudaDevAttrMultiProcessorCount, cfg->device);
     ctx->numa = numa_of_device(cfg->device);
     NumaScope numa_scope(ctx->numa);
     bool ok = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) == cudaSuccess;
@@ -1109,7 +1114,7 @@ int tad_init(const tad_config *cfg, tad_ctx **out)
     if (const char *e = getenv("TAD_EXCHANGE_CHUNKS")) ctx->exchange_chunks = atoi(e) < 1 ? 1 : (atoi(e) > kMaxXChunks ? kMaxXChunks : atoi(e));
     for (int i = 0; ok && i < kMaxEvents; i++) ok = cudaEventCreate(&ctx->ev[i]) == cudaSuccess;
     ok = ok && cudaHostAlloc((void **)&ctx->h_stats, 64 * sizeof(uint32_t), cudaHostAllocDefault) == cudaSuccess;
-    ok = ok && cudaHostAlloc((void **)&ctx->h_small, 256 * sizeof(unsigned long long), cudaHostAllocDefault) == cudaSuccess;
+    ok = ok && cudaHostAlloc((void **)&ctx->h_small, kSmallWords * sizeof(unsigned long long), cudaHostAllocDefault) == cudaSuccess;
     if (!ok) {
         tad_shutdown(ctx);      // releases whatever was created
         return TAD_ERR_CUDA;
@@ -1137,22 +1142,13 @@ void tad_shutdown(tad_ctx *ctx)
     if (ctx->worker.joinable()) ctx->worker.join();
     cudaSetDevice(ctx->cfg.device);
     if (ctx->peers_mapped && ctx->nccl.comm && ctx->small.p && ctx->stream) {
-        // an exported buffer must outlive every peer's mapping of it: unmap, meet the peers, only then free
+        // an exported buffer must outlive every peer's mapping of it: unmap, meet the peers, only then free (delete ctx)
         for (int r = 0; r < kMaxRanks; r++)
             if (ctx->peer_x[r]) { cudaIpcCloseMemHandle(ctx->peer_x[r]); ctx->peer_x[r] = nullptr; }
-        unsigned long long *d = static_cast<unsigned long long *>(ctx->small.p);
-        if (nccl_allgather(&ctx->nccl, d + 48, d + 56, 8, ctx->stream) == 0) cudaStreamSynchronize(ctx->stream);
+        if (barrier(ctx) == 0) cudaStreamSynchronize(ctx->stream);
         ctx->peers_mapped = false;
     }
     nccl_comm_destroy(&ctx->nccl);
-    DevBuf *bufs[] = {&ctx->xbuf, &ctx->xcnt, &ctx->xtotal, &ctx->sortb, &ctx->hist, &ctx->offsets, &ctx->cursor, &ctx->big_list, &ctx->big_base, &ctx->cls_list, &ctx->csr_p, &ctx->stats, &ctx->part, &ctx->csr_v,
-                      &ctx->csr_t, &ctx->nsb, &ctx->npb, &ctx->sbase, &ctx->outb, &ctx->ns_ignore, &ctx->spill, &ctx->dbx,
-                      &ctx->dbi, &ctx->exch, &ctx->scan_sync, &ctx->small, &ctx->hist_all, &ctx->seg_off, &ctx->seg_total,
-                      &ctx->entries, &ctx->ar_y, &ctx->ar_pred, &ctx->ar_lam, &ctx->ovf};
-    for (DevBuf *b : bufs)
-        if (b->p) cudaFree(b->p);
-    for (int i = 0; i < 10; i++)
-        if (ctx->d_col[i].p) cudaFree(ctx->d_col[i].p);
     for (auto &b : ctx->pinned_pool) cudaFreeHost(b.p);
     if (ctx->h_stats) cudaFreeHost(ctx->h_stats);
     if (ctx->h_small) cudaFreeHost(ctx->h_small);
@@ -1165,7 +1161,7 @@ void tad_shutdown(tad_ctx *ctx)
         if (ctx->x_ev[i]) cudaEventDestroy(ctx->x_ev[i]);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;      // frees the device workspace
 }
 
 int tad_alloc_columns(tad_ctx *ctx, uint64_t capacity, int32_t mem, tad_columns *cols)
